@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload arxiv|products|pubmed|cora]
     python bench.py --impl reference ...      # the CPU arm: oracle port on all host threads
+    python bench.py --dump-outputs DIR ...    # also write what the timed sweeps computed (one GPU; see dump_outputs)
 
 A "step" is one Jacobi sweep of Embedder.propagate (/root/reference/clane/embedder.py:84-108)
 over the whole graph with P frozen: the fused gather-SpMM + residual kernel(s), the exact
@@ -44,7 +45,14 @@ def parse_args():
     ap.add_argument("--scale", type=float, default=1.0, help="shrink the workload (debug only; marks the line invalid)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-converge", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (single-GPU arm; see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "clane_b200":
+        ap.error("--dump-outputs writes the outputs of the GPU arm")
+    return args
 
 
 def workload_name(args) -> str:
@@ -65,6 +73,31 @@ def workload_config(name, n, e, d, scale):
 def sweep_bytes(n, e, d):
     """Algorithmic bytes of one sweep (SURVEY.md 8d): X, Z_cur read, Z_next written, col, w, rowptr."""
     return 12 * d * n + 8 * e + 4 * (n + 1)
+
+
+DUMP_Z_BYTES = 32 << 20
+
+
+def dump_outputs(out_dir, S, steps):
+    """What the timed sweeps computed, as a caller of Embedder.propagate receives it, so that two builds can be compared
+    output for output.  All sweeps of a run, warm-up (the line's `warmup` counts them) and timed, are one sequence from
+    Z = X with P built from X, so the same arguments give the same outputs:
+
+        Z.npy        float32 [rows, d]  embeddings after the last timed sweep: every row, or, when Z is larger than
+                                        DUMP_Z_BYTES, a fixed sample of rows (seed 0, ascending)
+        Z_rows.npy   float64 [rows]     the row ids of Z.npy
+        amounts.npy  float32 [steps]    the exact L1 change of every timed sweep, the last one last"""
+    import torch
+    n, d = S.n, S.d
+    rows = np.arange(n)
+    if n * d * 4 > DUMP_Z_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(n, DUMP_Z_BYTES // (4 * d), replace=False))
+    Z = S.Z[S.cur][torch.from_numpy(rows).to(S.device), :d].cpu().numpy()
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    np.save(out / "Z.npy", Z)
+    np.save(out / "Z_rows.npy", rows.astype(np.float64))
+    np.save(out / "amounts.npy", S.log[:steps].cpu().numpy())
 
 
 def measured_peak():
@@ -297,6 +330,8 @@ def run_gpu(args):
     emb.verbose = False
 
     if world > 1:
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs writes the outputs of a single-GPU run")
         from clane_b200 import dist as cdist
         runner = cdist.ShardedSweeper(g, sim, GAMMA, exchange=os.environ.get("CLANE_EXCHANGE", "auto"))
         S = None
@@ -304,6 +339,8 @@ def run_gpu(args):
         runner = None
         S = g._device_state()
         g._build_P_device(sim)
+        if args.dump_outputs and args.steps > S.log_cap:
+            raise SystemExit(f"--dump-outputs keeps the L1 change of at most {S.log_cap} timed sweeps")
     stream = S.stream if S is not None else torch.cuda.current_stream()
     torch.cuda.synchronize()
     sh = stream.cuda_stream
@@ -389,6 +426,8 @@ def run_gpu(args):
     sampler = ClockSampler(local_rank)
     sampler.start()
     total_ms = timed_loop(args.steps)                                  # the metric: whole steps
+    if args.dump_outputs:                                              # before kernel_loop overwrites the Z buffers
+        dump_outputs(args.dump_outputs, S, args.steps)
     kern = kernel_loop(min(args.steps, 200))                           # per-kernel durations (roofline)
     phases = None
     exch = runner.exchange if runner is not None else "none"

@@ -687,6 +687,35 @@ def test_value_finish_small_and_ragged(n, d):
     assert np.float32(out.cpu().numpy()[0]) == O.l1_diff(a, b)
 
 
+@pytest.mark.parametrize("shape", ["cora", "arxiv"])
+def test_bench_dump_outputs_are_the_timed_sweeps(shape, tmp_path):
+    """bench.py --dump-outputs: the warm-up and timed sweeps are one sequence from Z = X, so Z after the last timed
+    sweep and the L1 change of each timed sweep equal the oracle's propagate() of warmup + steps sweeps, bit-exact;
+    arxiv's Z is larger than the dump's budget and is sampled."""
+    import json
+    import subprocess
+    import sys
+    steps = 7
+    cmd = [sys.executable, str(ROOT / "bench.py"), "--workload", shape, "--steps", str(steps), "--warmup", "2",
+           "--no-cpu-baseline", "--no-converge", "--dump-outputs", str(tmp_path)]
+    r = subprocess.run(cmd, capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
+    line = json.loads([ln for ln in r.stdout.split("\n") if ln.startswith("{")][-1])
+    assert line["steps"] == steps and line["warmup"] >= 2
+    assert sum(p.stat().st_size for p in tmp_path.iterdir()) <= 64 << 20
+    n, src, dst, X = synth.make_graph(shape, seed=0)
+    O.set_threads(O.max_threads())
+    rowptr, col = O.csr_from_edges(src, dst, n)
+    Zo, amounts, _ = O.propagate(X, X, rowptr, col, 0.76, 1 << 30, max_sweeps=line["warmup"] + steps)
+    amounts = amounts[-steps:]
+    rows = np.load(tmp_path / "Z_rows.npy")
+    assert rows.dtype == np.float64 and np.all(np.diff(rows) > 0)
+    assert len(rows) == (n if shape == "cora" else 65536)
+    Z = np.load(tmp_path / "Z.npy")
+    assert Z.dtype == np.float32 and np.array_equal(Z, Zo[rows.astype(np.int64)])
+    assert np.array_equal(np.load(tmp_path / "amounts.npy"), amounts) and len(amounts) == steps
+
+
 def test_sharded_run_equals_single_gpu_when_two_gpus_are_present():
     """tools/check_dist.py under torchrun (2 ranks, fused peer-store exchange): bit-identical to the single-GPU
     run at four shapes.  Skipped on a one-GPU box."""
