@@ -368,11 +368,11 @@ __device__ __noinline__ void restage_meta(const SweepParams& p, int lane, int2* 
 // Span task: a run of consecutive ordinary rows of one row group (a whole group when `direct`), one row at a time:
 // the row's X piece, its own Zcur piece (fused L1) and <= 8 gathers are issued together and reduced in the
 // reference's order -- one memory round trip per 8 neighbours.  No descriptors: the degrees come from rowptr (lane r
-// holds row r0 + r), the edges from the staged window.  The gathers are 128-bit loads straight into registers;
-// X and the own piece go through cp.async into 1 KB of the warp's shared memory, so that the 8 registers they
-// would occupy while the gathers are in flight are free: the kernel fits 64 registers = 32 resident warps per SM,
-// each with one batch of loads in flight (tools/l1pf_probe.cu: resident warps beat deeper per-warp pipelines on
-// this access pattern).
+// holds the degree of row r0 + r, r < nrows <= 32), the edges from the staged window.  The gathers are 128-bit
+// loads straight into registers; X and the own piece go through cp.async into 1 KB of the warp's shared memory, so
+// that the 8 registers they would occupy while the gathers are in flight are free: the kernel fits 64 registers = 32
+// resident warps per SM, each with one batch of loads in flight (tools/l1pf_probe.cu: resident warps beat deeper
+// per-warp pipelines on this access pattern).
 template <bool kBulk>
 __device__ __forceinline__ void run_span(const SweepParams& p, const int4 t0, int slab, int lane, int2* meta, float* scratch,
                                          float4* rowbuf, int* state, float* stage) {
@@ -383,10 +383,13 @@ __device__ __forceinline__ void run_span(const SweepParams& p, const int4 t0, in
     const int cc = active ? c0 : 0;            // idle lanes shadow lane 0 (same sectors: no extra traffic)
     const bool col_blocked = cc < p.limit;
     const bool all_blocked = p.limit == p.ld;  // uniform
+    // lane r: the degree of row r0 + r from its own pair of rowptr entries (same line).  A span has up to 32 rows, so
+    // lane 31 has no lane 32 to take its row's end from; lanes past the span read rowptr[r0 + nrows] twice (degree 0)
     const int rp = __ldg(p.rowptr + r0 + min(lane, nrows));
+    const int rp_next = __ldg(p.rowptr + r0 + min(lane + 1, nrows));
     if (lane == 0) { state[0] = t0.x; state[1] = t0.y; }
     stage_meta(p, t0.x, t0.y, lane, meta);
-    const int deg = __shfl_down_sync(kFull, rp, 1) - rp;
+    const int deg = rp_next - rp;
     const float4* zb = reinterpret_cast<const float4*>(p.Zc + cc);
     const unsigned rowbuf_sa = smem_u32(rowbuf + lane);
     const int nseg = p.d >> 5;
@@ -604,22 +607,26 @@ __global__ void __launch_bounds__(kChainThreads, kLight ? 16 : 1) k_hub_chain(Sw
     constexpr int kTailPitch = kTailGroup + 4;
     extern __shared__ __align__(16) unsigned char smem[];
     __shared__ unsigned long long full[kMaxStages], empty[kMaxStages];
+    __shared__ int stop;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int per = p.nslab32b + (p.ntail4 > 0 ? 1 : 0);
     const int hr = p.hub_first + blockIdx.x / per, s = blockIdx.x % per;
-    if (p.st != nullptr && p.st->stop) return;
-    trace_begin(p.trace);
     const int4 info = __ldg(p.hub_info + hr);
     const int row = info.x, a = info.y, k = info.z;
     const int nblk = k >> 3;
     const size_t B0 = (size_t)info.w;
     const int nleft = k - nblk * 8;
     if (threadIdx.x == 0) {
+        // one read of the flag for the whole CTA: the tail of the previous sweep may set it while this (speculative)
+        // sweep runs, and a producer warp that returned while the chain warp went on would leave it waiting forever
+        stop = p.st != nullptr && p.st->stop;
 #pragma unroll
         for (int i = 0; i < kMaxStages; ++i) { mbar_init(full + i, 32); mbar_init(empty + i, 1); }   // (unrolled: ~0.3 us)
         fence_mbar_init();
     }
     __syncthreads();
+    if (stop) return;
+    trace_begin(p.trace);
     const bool blocked = s < p.nslab32b;
     const int nt = p.ntail4, ntc = p.ld - p.limit;                  // sequential-regime float4 pieces / columns
     const int nnb = nblk * 8;

@@ -217,6 +217,34 @@ def test_group_schedule_degree_sorted_row_blocks():
     assert group_schedule(rp, 140000, 100, 0, 140000)[4:] == (8, False)
 
 
+@pytest.mark.parametrize("d", [32, 64, 128])
+def test_group_schedule_fused_group_size_at_the_level_step_boundaries(d):
+    """A fused group is one level-0 chunk of the L1 cascade over n*d (32 * level step elements): the step goes from
+    16 to 32 above n*d = 2^24 and from 32 to 64 above 2^28, where the chunk outgrows a warp's 1024 floats and fusion
+    turns off."""
+    for elems, G, fused in [(1 << 24, 512 // d, True), ((1 << 24) + d, 1024 // d, True),
+                            (1 << 28, 1024 // d, True), ((1 << 28) + d, 8, False)]:
+        n = elems // d
+        assert group_schedule(np.zeros(n + 1, np.int32), n, d, 0, n)[4:] == (G, fused), (n, d)
+
+
+def test_group_schedule_direct_32_row_spans():
+    """d = 32 above 2^24 elements: 32-row groups, and a low-degree graph sweeps every group as one direct span --
+    lane 31 of the warp holds a row of its own."""
+    rng = np.random.default_rng(17)
+    n, d = 600000, 32
+    rowptr = np.concatenate([[0], np.cumsum(rng.integers(1, 5, n))]).astype(np.int32)
+    sr, sm, fx, hr, G, fused = group_schedule(rowptr, n, d, 0, n, 256)
+    assert (G, fused) == (32, True) and len(fx) == 0 and len(hr) == 0
+    assert np.array_equal(np.sort(sr), np.arange(0, n, 32)) and np.all(sm == 32 | (1 << 8))
+    tasks = sweep_program(rowptr, n, d, 0, n, 256)
+    assert len(tasks) == n // 32 and np.all(tasks[:, 3] == 32 | (1 << 8))
+    for t in tasks[::997]:
+        _, direct, out = emulate_task(t, rowptr)
+        assert direct and [r for r, _ in out] == list(range(t[2], t[2] + 32))
+        assert out[31][1] == list(range(rowptr[t[2] + 31], rowptr[t[2] + 32]))
+
+
 def test_cascade_shape():
     L = _lib.lib()
     nodes, per = ctypes.c_int64(), ctypes.c_int64()
@@ -328,9 +356,11 @@ def emulate_task(task, rowptr):
     if segment:        # whole (offset, w) stream in the window, batches of 8 in order
         assert e_total <= 128 and e_total == 8 * nb and r0 + nb <= nblk_row
         return True, False, [(blk_base + r0 + b, list(range(e_first + 8 * b, e_first + 8 * b + 8))) for b in range(nb)]
-    # span: degrees from rowptr (lane r holds row r0 + r), a 128-entry window of the edge stream, restaged when a
-    # batch starts at its end (only a single row longer than the window gets there)
+    # span: lane l takes the degree of row r0 + l from rowptr[r0 + min(l, nrows)] and rowptr[r0 + min(l + 1, nrows)]
+    # (lanes past the span: 0), a 128-entry window of the edge stream, restaged when a batch starts at its end (only a
+    # single row longer than the window gets there)
     assert 1 <= nrows <= 32 and e_first == rowptr[r0] and e_total == rowptr[r0 + nrows] - e_first
+    lane_deg = [int(rowptr[r0 + min(lane + 1, nrows)] - rowptr[r0 + min(lane, nrows)]) for lane in range(32)]
     nonsink = sum(1 for r in range(nrows) if rowptr[r0 + r + 1] > rowptr[r0 + r])
     assert e_total <= 128 or nonsink == 1          # a row longer than the window is the only row with edges in its span
     state = [e_first, e_total]
@@ -351,7 +381,7 @@ def emulate_task(task, rowptr):
         return got
 
     for r in range(nrows):
-        k = int(rowptr[r0 + r + 1] - rowptr[r0 + r])
+        k = lane_deg[r]
         if k == 0:
             continue
         cur = []
