@@ -25,6 +25,12 @@ class Patience(C.Structure):
                 ("max_sweeps", C.c_int32), ("stop", C.c_int32), ("last_amount", C.c_float), ("reserved", C.c_int32)]
 
 
+class Patience64(C.Structure):
+    """Mirror of ``struct clane_patience64`` (40 bytes)."""
+    _fields_ = [("minimum", C.c_double), ("last_amount", C.c_double), ("patience", C.c_int32), ("tol", C.c_int32),
+                ("sweeps", C.c_int32), ("max_sweeps", C.c_int32), ("stop", C.c_int32), ("reserved", C.c_int32)]
+
+
 CLANE_EUNSUPPORTED = -9
 
 
@@ -78,6 +84,17 @@ SIGNATURES = {
     "clane_plan_profile": (C.c_int, [c_vp, C.c_int]),
     "clane_plan_profile_read": (C.c_int, [c_vp, c_f32p]),
     "clane_patience_reset": (C.c_int, [c_vp, C.c_int32, C.c_int32, c_vp]),
+    "clane_padded_ld_f64": (C.c_int32, [C.c_int32]),
+    "clane_work_f64": (C.c_int64, [C.c_int64]),
+    "clane_patience_reset_f64": (C.c_int, [c_vp, C.c_int32, C.c_int32, c_vp]),
+    "clane_l1_diff_f64": (C.c_int, [C.c_int32, C.c_int32, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    "clane_row_softmax_f64": (C.c_int, [c_vp, c_vp, C.c_int32, C.c_int32, c_vp, c_vp, c_vp]),
+    "clane_build_p_cosine_f64": (C.c_int, [C.c_int32, C.c_int64, C.c_int32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,
+                                           c_vp]),
+    "clane_sweep_f64": (C.c_int, [C.c_int32, C.c_int32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, C.c_double, c_vp, c_vp, c_vp,
+                                  C.c_int32, c_vp, c_vp]),
+    "clane_sweeps_f64": (C.c_int, [C.c_int32, C.c_int32, c_vp, c_vp, c_vp, c_vp, c_vp, C.c_int32, C.c_double, C.c_int32,
+                                   c_vp, c_vp, C.c_int32, c_vp, c_vp]),
     "clane_session_create": (C.c_int, [C.POINTER(c_vp), C.c_int32, C.c_int64, C.c_int32, c_vp, c_vp, c_vp, C.c_int32]),
     "clane_session_destroy": (C.c_int, [c_vp]),
     "clane_session_set_z": (C.c_int, [c_vp, c_vp]),

@@ -117,6 +117,9 @@ class ShardedSweeper:
     """Sweeps of one propagate() call over this rank's rows, with the per-sweep exchange."""
 
     def __init__(self, graph, similarity, gamma: float, tol: int = 10, max_sweeps: int = 0, exchange: str = "auto"):
+        if graph.X.dtype != torch.float32:
+            raise NotImplementedError(f"sharded sweeps run in fp32 only; content embeddings are {graph.X.dtype} "
+                                      "(use Embedder on one GPU for fp64)")
         self.g, self.sim, self.gamma = graph, similarity, float(np.float32(gamma))
         self.world, self.rank = dist.get_world_size(), dist.get_rank()
         self.dev = _lib.require_cuda()

@@ -48,11 +48,11 @@ class HistoryWriter(object):
     /root/reference/clane/__main__.py:73-82) while the sweeps run: each sweep's Z goes device -> one of three pinned
     host buffers -> a writer thread, instead of accumulating N*d*4 bytes per sweep in host memory until the end."""
 
-    def __init__(self, root: Path, n: int, d: int) -> None:
+    def __init__(self, root: Path, n: int, d: int, dtype: torch.dtype = torch.float32) -> None:
         self.root = Path(root)
         self.free, self.work = queue.Queue(), queue.Queue()
         for _ in range(3):
-            self.free.put(torch.empty([n, d], dtype=torch.float32).pin_memory())
+            self.free.put(torch.empty([n, d], dtype=dtype).pin_memory())
         self.error = None
         self.thread = threading.Thread(target=self._run, daemon=True)
         self.thread.start()
@@ -139,7 +139,7 @@ class Embedder(object):
         S = g._device_state()
         prev = torch.empty_like(S.Z[0])
         if self.save_history and self.history_root is not None:
-            self._history_writer = HistoryWriter(self.history_root, S.n, S.d)
+            self._history_writer = HistoryWriter(self.history_root, S.n, S.d, S.dtype)
         try:
             self._iterate(g, L, S, prev)
         finally:
@@ -151,8 +151,12 @@ class Embedder(object):
         while True:
             prev.copy_(S.Z[S.cur])
             self.propagate()
-            _lib.check(L.clane_l1_diff(S.plan.handle, S.Z[S.cur].data_ptr(), prev.data_ptr(), S.amount.data_ptr(),
-                                       _lib.stream_handle()), "clane_l1_diff")
+            if S.dtype == torch.float64:
+                _lib.check(L.clane_l1_diff_f64(S.n, S.d, S.Z[S.cur].data_ptr(), prev.data_ptr(), S.work.data_ptr(),
+                                               S.amount.data_ptr(), _lib.stream_handle()), "clane_l1_diff_f64")
+            else:
+                _lib.check(L.clane_l1_diff(S.plan.handle, S.Z[S.cur].data_ptr(), prev.data_ptr(), S.amount.data_ptr(),
+                                           _lib.stream_handle()), "clane_l1_diff")
             amount_updated_Z_current = float(S.amount.cpu()[0])   # synchronises the current stream
             if self.minimum_amount_updated_Z > amount_updated_Z_current:
                 self.tolerences['global'].reset()
@@ -176,9 +180,15 @@ class Embedder(object):
         caller = torch.cuda.current_stream()
         S.stream.wait_stream(caller)
         stream = S.stream.cuda_stream
-        _lib.check(L.clane_patience_reset(S.state.data_ptr(), int(tol.initial_value), int(max_sweeps), stream),
-                   "clane_patience_reset")
-        gamma = ctypes.c_float(float(np.float32(self.gamma)))
+        f64 = S.dtype == torch.float64
+        if f64:
+            _lib.check(L.clane_patience_reset_f64(S.state.data_ptr(), int(tol.initial_value), int(max_sweeps), stream),
+                       "clane_patience_reset_f64")
+            gamma = ctypes.c_double(float(self.gamma))     # gamma scales a double tensor: not rounded to fp32
+        else:
+            _lib.check(L.clane_patience_reset(S.state.data_ptr(), int(tol.initial_value), int(max_sweeps), stream),
+                       "clane_patience_reset")
+            gamma = ctypes.c_float(float(np.float32(self.gamma)))
         history_Z = [] if self.save_history else None
         start = S.cur
 
@@ -186,9 +196,17 @@ class Embedder(object):
             with torch.cuda.stream(S.stream):
                 S.state_host.copy_(S.state, non_blocking=True)
             S.stream.synchronize()
-            return _lib.Patience.from_buffer_copy(S.state_host.numpy().tobytes())
+            return (_lib.Patience64 if f64 else _lib.Patience).from_buffer_copy(S.state_host.numpy().tobytes())
 
-        if history_Z is None:
+        if f64 and history_Z is None:
+            # batches of sweeps enqueued directly, one sync each; sweeps past the stop are device-side no-ops
+            st = None
+            while st is None or not st.stop:
+                _lib.check(L.clane_sweeps_f64(S.n, S.d, S.rowptr.data_ptr(), S.col.data_ptr(), S.w.data_ptr(),
+                                              S.X.data_ptr(), S.Zptrs, start, gamma, 12, S.state.data_ptr(),
+                                              S.log.data_ptr(), S.log_cap, S.work.data_ptr(), stream), "clane_sweeps_f64")
+                st = read_state()    # 12 sweeps = whole rotations: every batch starts at the same buffer
+        elif history_Z is None:
             # the whole call is ONE graph launch: a conditional WHILE node repeats batches of sweeps (the L1 / patience
             # tail of every sweep beside the rows of the next one) until the device-side patience counter hits zero
             rc = L.clane_sweeps(S.plan.handle, S.X.data_ptr(), S.Zptrs, start, S.rowptr.data_ptr(), S.col.data_ptr(),
@@ -208,9 +226,15 @@ class Embedder(object):
             k = 0
             while True:
                 src, dst = S.Z[(start + k) % 3], S.Z[(start + k + 1) % 3]
-                _lib.check(L.clane_sweep(S.plan.handle, S.X.data_ptr(), src.data_ptr(), dst.data_ptr(),
-                                         S.rowptr.data_ptr(), S.col.data_ptr(), S.w.data_ptr(), gamma,
-                                         0, S.state.data_ptr(), S.log.data_ptr(), S.log_cap, stream), "clane_sweep")
+                if f64:
+                    _lib.check(L.clane_sweep_f64(S.n, S.d, S.rowptr.data_ptr(), S.col.data_ptr(), S.w.data_ptr(),
+                                                 S.X.data_ptr(), src.data_ptr(), dst.data_ptr(), gamma, None,
+                                                 S.state.data_ptr(), S.log.data_ptr(), S.log_cap, S.work.data_ptr(),
+                                                 stream), "clane_sweep_f64")
+                else:
+                    _lib.check(L.clane_sweep(S.plan.handle, S.X.data_ptr(), src.data_ptr(), dst.data_ptr(),
+                                             S.rowptr.data_ptr(), S.col.data_ptr(), S.w.data_ptr(), gamma,
+                                             0, S.state.data_ptr(), S.log.data_ptr(), S.log_cap, stream), "clane_sweep")
                 k += 1
                 st = read_state()
                 if self._history_writer is not None:

@@ -8,6 +8,7 @@ on every access) and everything the iterative update touches lives in HBM:
 
     rowptr int32[N+1] | col int32[E] | erow int32[E] | w fp32[E]
     X fp32[N, ld] | Z fp32[3][N, ld]   (ld = d rounded up to 4 floats: 16-byte aligned rows; three rotating buffers)
+    (float64 features: w, X and Z are fp64 with ld = d rounded up to 2, and the update runs in double, DESIGN.md 7b)
     clane_plan: the degree-sorted row-block schedule (hub groups / row groups, sinks dropped)
 
 All arithmetic is done by libclane_b200.so through the C-ABI (clane_b200/_lib.py); torch
@@ -213,31 +214,39 @@ class Graph(Dataset):
     def _device_state(self):
         if self._dev is None:
             dev = _lib.require_cuda()
-            if self.X.dtype != torch.float32:
+            if self.X.dtype not in (torch.float32, torch.float64):
                 raise NotImplementedError(
-                    f"clane_b200 computes in fp32; content embeddings are {self.X.dtype} "
+                    f"clane_b200 computes in fp32 or fp64; content embeddings are {self.X.dtype} "
                     "(the reference would run its whole update in that dtype, graph.py:51)")
             L = _lib.lib()
             n, e, d = self._n, self._nnz, int(self.X.shape[1])
-            ld = int(L.clane_padded_ld(d))
             S = type("DeviceState", (), {})()
+            S.dtype = self.X.dtype
+            f64 = S.dtype == torch.float64
+            ld = int(L.clane_padded_ld_f64(d) if f64 else L.clane_padded_ld(d))
             S.device, S.n, S.e, S.d, S.ld = dev, n, e, d, ld
             S.rowptr = torch.from_numpy(self._rowptr).to(dev)
             S.col = torch.from_numpy(self._col if e else np.zeros(1, np.int32)).to(dev)
             S.erow = torch.zeros(max(e, 1), dtype=torch.int32, device=dev)
-            S.plan = _lib.Plan(n, e, d, self._rowptr, 0, n, HUB_THRESHOLD)   # module attribute: tests lower it
-            S.X = torch.zeros([max(n, 1), ld], dtype=torch.float32, device=dev)
+            # fp64 runs without a plan: its kernels take plain sizes and the reduction scratch S.work
+            S.plan = None if f64 else _lib.Plan(n, e, d, self._rowptr, 0, n, HUB_THRESHOLD)   # module attribute: tests lower it
+            S.X = torch.zeros([max(n, 1), ld], dtype=S.dtype, device=dev)
             S.X[:n, :d] = self.X.to(dev)
             S.Z = [torch.zeros_like(S.X) for _ in range(3)]     # rotating: sweep t reads Z[(cur + t) % 3], writes the next
             S.Zptrs = (ctypes.c_void_p * 3)(*[z.data_ptr() for z in S.Z])
             S.cur = 0
-            S.w = torch.zeros(max(e, 1), dtype=torch.float32, device=dev)
-            S.norms2 = torch.zeros(2, dtype=torch.float32, device=dev)
-            S.amount = torch.zeros(1, dtype=torch.float32, device=dev)
-            S.state = torch.zeros(8, dtype=torch.int32, device=dev)          # struct clane_patience
-            S.state_host = torch.zeros(8, dtype=torch.int32).pin_memory()
+            S.w = torch.zeros(max(e, 1), dtype=S.dtype, device=dev)
+            S.norms2 = torch.zeros(2, dtype=S.dtype, device=dev)
+            S.amount = torch.zeros(1, dtype=S.dtype, device=dev)
+            if f64:
+                S.state = torch.zeros(ctypes.sizeof(_lib.Patience64), dtype=torch.uint8, device=dev)
+                S.state_host = torch.zeros(ctypes.sizeof(_lib.Patience64), dtype=torch.uint8).pin_memory()
+                S.work = torch.zeros(int(L.clane_work_f64(max(n * d, e * d))), dtype=torch.float64, device=dev)
+            else:
+                S.state = torch.zeros(8, dtype=torch.int32, device=dev)          # struct clane_patience
+                S.state_host = torch.zeros(8, dtype=torch.int32).pin_memory()
             S.log_cap = 1 << 16
-            S.log = torch.zeros(S.log_cap, dtype=torch.float32, device=dev)
+            S.log = torch.zeros(S.log_cap, dtype=S.dtype, device=dev)
             S.stream = torch.cuda.Stream(device=dev)   # sweeps run here (a capturable stream: CUDA-graph replay)
             _lib.check(L.clane_edge_rows(S.rowptr.data_ptr(), n, e, S.erow.data_ptr(), _lib.stream_handle()),
                        "clane_edge_rows")
@@ -250,7 +259,7 @@ class Graph(Dataset):
         if tuple(Z.shape) != (S.n, S.d):
             raise ValueError(f"Z has shape {tuple(Z.shape)}, expected {(S.n, S.d)}")
         S.Z[0].zero_()
-        S.Z[0][:S.n, :S.d] = Z.to(device=S.device, dtype=torch.float32)
+        S.Z[0][:S.n, :S.d] = Z.to(device=S.device, dtype=S.dtype)
         S.Z[1].copy_(S.Z[0])
         S.Z[2].copy_(S.Z[0])
         S.cur = 0
@@ -284,7 +293,7 @@ class Graph(Dataset):
             self._Z_host[idx] = value.to(self._Z_host.dtype)
         else:
             S = self._dev
-            row = value.to(device=S.device, dtype=torch.float32).reshape(S.d)
+            row = value.to(device=S.device, dtype=S.dtype).reshape(S.d)
             for z in S.Z:                       # every buffer: rows without out-neighbours are never rewritten by a sweep
                 z[idx, :S.d] = row
 
@@ -303,6 +312,8 @@ class Graph(Dataset):
         L = _lib.lib()
         Zc = S.Z[S.cur]
         stream = _lib.stream_handle()
+        if S.dtype == torch.float64:
+            return self._build_P_device_f64(similarity, S, L, Zc, stream)
         if getattr(similarity, "_clane_kernel", None) == "cosine":
             _lib.check(L.clane_build_p_cosine(S.plan.handle, Zc.data_ptr(), S.rowptr.data_ptr(), S.erow.data_ptr(),
                                               S.col.data_ptr(), S.w.data_ptr(), S.norms2.data_ptr(), stream),
@@ -327,6 +338,23 @@ class Graph(Dataset):
                 raise ValueError(f"similarity returned {scores.numel()} scores for {S.e} edges")
             _lib.check(L.clane_row_softmax(scores.data_ptr(), 0, 0, S.n, S.rowptr.data_ptr(), S.w.data_ptr(), stream),
                        "clane_row_softmax")
+        return S.w[:S.e]
+
+    def _build_P_device_f64(self, similarity, S, L, Zc, stream) -> torch.Tensor:
+        """build_P in double: cosine on the fused fp64 kernels; any other scorer (the trainable asymmetric one
+        included, whose fp32 weights then raise torch's dtype error as upstream) scores in double as a plugin."""
+        if getattr(similarity, "_clane_kernel", None) == "cosine":
+            _lib.check(L.clane_build_p_cosine_f64(S.n, S.e, S.d, Zc.data_ptr(), S.rowptr.data_ptr(), S.erow.data_ptr(),
+                                                  S.col.data_ptr(), S.w.data_ptr(), S.norms2.data_ptr(),
+                                                  S.work.data_ptr(), stream), "clane_build_p_cosine_f64")
+        else:
+            Zv = Zc[:S.n, :S.d]
+            src_Z, dst_Z = Zv[S.erow[:S.e].long()], Zv[S.col[:S.e].long()]
+            scores = similarity(src_Z, dst_Z).detach().to(device=S.device, dtype=torch.float64).reshape(-1).contiguous()
+            if scores.numel() != S.e:
+                raise ValueError(f"similarity returned {scores.numel()} scores for {S.e} edges")
+            _lib.check(L.clane_row_softmax_f64(scores.data_ptr(), None, 0, S.n, S.rowptr.data_ptr(), S.w.data_ptr(),
+                                               stream), "clane_row_softmax_f64")
         return S.w[:S.e]
 
     def build_P(self, similarity) -> torch.Tensor:

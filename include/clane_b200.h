@@ -293,6 +293,60 @@ int clane_plan_profile_read(clane_plan* plan, float* h_ms);
 /* Reset the device patience state for a new propagate() call (embedder.py:78-79). */
 int clane_patience_reset(clane_patience* d_state, int32_t tol, int32_t max_sweeps, clane_stream_t s);
 
+/* ---- float64 ------------------------------------------------------------------------- */
+/* When the content embeddings are float64 the reference runs build_P, every sweep, the L1 change and
+ * both patience loops in double (graph.py:51 keeps the dtype of C.npy).  These entry points reproduce
+ * that run bit for bit (DESIGN.md, "fp64"): the row update is one sequential fma chain over the
+ * neighbours for every column, torch.sum is the ATen cascade with 4 lanes x 4 ILP rows, softmax(0) is
+ * Sleef expd u10 with an 8-lane reduce_all.  They take plain sizes instead of a clane_plan:
+ *   - feature matrices are row-major fp64 [n, ld] with ld = clane_padded_ld_f64(d) (rows 16-byte
+ *     aligned); the pad columns must be zero and stay zero;
+ *   - d_work is caller-owned device scratch of clane_work_f64(m) doubles, m the largest reduction it
+ *     serves: n * d for the sweeps and clane_l1_diff_f64, e * d for clane_build_p_cosine_f64. */
+typedef struct clane_patience64 {
+    double  minimum;      /* running strict minimum of the per-sweep L1 amount (starts +inf) */
+    double  last_amount;  /* L1 amount of the last completed sweep                           */
+    int32_t patience;     /* as in clane_patience                                             */
+    int32_t tol;
+    int32_t sweeps;
+    int32_t max_sweeps;
+    int32_t stop;
+    int32_t reserved;
+} clane_patience64;
+
+/* d rounded up to a multiple of 2 */
+int32_t clane_padded_ld_f64(int32_t d);
+/* doubles of d_work that suffice for every reduction over at most n_elems elements (non-decreasing in
+ * n_elems, so one buffer sized for the largest reduction serves the smaller ones) */
+int64_t clane_work_f64(int64_t n_elems);
+/* clane_patience_reset for the float64 state */
+int clane_patience_reset_f64(clane_patience64* d_state, int32_t tol, int32_t max_sweeps, clane_stream_t s);
+/* (Za - Zb).abs().sum() over the flattened [n*d] array (embedder.py:60) -> d_out[0] */
+int clane_l1_diff_f64(int32_t n, int32_t d, const double* d_Za, const double* d_Zb, double* d_work, double* d_out,
+                      clane_stream_t s);
+/* clane_row_softmax in double; for scores a user plugin produced, pass d_norms2 = NULL.  d_w may alias d_scores. */
+int clane_row_softmax_f64(const double* d_scores, const double* d_norms2, int32_t row_lo, int32_t row_hi,
+                          const int32_t* d_rowptr, double* d_w, clane_stream_t s);
+/* Graph.build_P with CosineSimilarity in double: per-edge dots, the two global norms (d_norms2[0..1]),
+ * the division and the row softmax -> d_w[e]. */
+int clane_build_p_cosine_f64(int32_t n, int64_t e, int32_t d, const double* d_Z, const int32_t* d_rowptr,
+                             const int32_t* d_erow, const int32_t* d_col, double* d_w, double* d_norms2,
+                             double* d_work, clane_stream_t s);
+/* clane_sweep in double: Znext[v] = X[v] + gamma * (w_v @ Zcur[nbrs(v)]) for rows with out-neighbours;
+ * the L1 change to d_amount (if not NULL) and the patience step (if d_state is not NULL; a no-op once
+ * d_state->stop is set). */
+int clane_sweep_f64(int32_t n, int32_t d, const int32_t* d_rowptr, const int32_t* d_col, const double* d_w,
+                    const double* d_X, const double* d_Zcur, double* d_Znext, double gamma, double* d_amount,
+                    clane_patience64* d_state, double* d_amounts_log, int32_t log_cap, double* d_work,
+                    clane_stream_t s);
+/* n_sweeps sweeps enqueued at once with the patience state on the device: sweep t reads d_Z3[(cur + t) % 3]
+ * and writes d_Z3[(cur + t + 1) % 3].  Sweeps after the stop are device-side no-ops, so the caller polls
+ * d_state once per batch; the result is d_Z3[(cur + d_state->sweeps) % 3]. */
+int clane_sweeps_f64(int32_t n, int32_t d, const int32_t* d_rowptr, const int32_t* d_col, const double* d_w,
+                     const double* d_X, double* const* d_Z3, int32_t cur, double gamma, int32_t n_sweeps,
+                     clane_patience64* d_state, double* d_amounts_log, int32_t log_cap, double* d_work,
+                     clane_stream_t s);
+
 /* ---- host-buffer session API (pure C consumers; bench e2e) ---------------------------- */
 typedef struct clane_session clane_session;
 
