@@ -261,7 +261,7 @@ int clane_plan_destroy(clane_plan* plan) {
     cudaFree(plan->d_P0); cudaFree(plan->d_coloff); cudaFree(plan->d_trace);
     for (auto& g : plan->graphs) if (g.exec) cudaGraphExecDestroy(g.exec);
     for (int i = 0; i < 8; ++i) if (plan->ev_prof[i]) cudaEventDestroy(plan->ev_prof[i]);
-    cudaFree(plan->d_p1); cudaFree(plan->d_p2); cudaFree(plan->d_p0n);
+    cudaFree(plan->d_p1); cudaFree(plan->d_p2);
     delete plan;
     return CLANE_OK;
 }
@@ -361,12 +361,6 @@ int clane_plan_create(clane_plan** out, int32_t n, int64_t e, int32_t d, const i
     const int64_t auto_thr = std::min<int64_t>(16384, std::max<int64_t>(256, (e_local / 4096 + 7) / 8 * 8));
     plan->hub_threshold = hub_threshold > 0 ? std::min(std::max(hub_threshold, 8), 1 << 20) : (int32_t)auto_thr;
     plan->span_edges = 128;
-    // measured at arxiv shape: a propagate() of 20 sweeps is 1.2 ms faster enqueued directly (no graph to build), but a
-    // host-driven loop stalls the device at every state read; so direct enqueue stays an opt-in
-    plan->prefer_direct = getenv("CLANE_PREFER_DIRECT") != nullptr;
-    // tuning aids (benchmark sweeps only)
-    if (const char* v = getenv("CLANE_HUB_THRESHOLD")) plan->hub_threshold = std::max(atoi(v), 8);
-    if (const char* v = getenv("CLANE_SPAN_EDGES")) plan->span_edges = std::min(std::max(atoi(v), 8), clane::kMetaRing);
     plan->nslab = (plan->ld + 127) / 128;
     plan->limit = (d / 16) * 16;
     plan->ntail4 = (plan->ld - plan->limit) / 4;
@@ -632,8 +626,7 @@ int clane_session_propagate(clane_session* s, float gamma, int32_t tol, int32_t 
     // batches of 12 sweeps (whole buffer rotations), one host synchronisation per batch
     // ... except for a short bounded call (max_sweeps <= 24): its sweeps are enqueued directly, once -- no graph to build,
     // the device-side counter turns whatever follows the stop into no-ops
-    static const bool no_direct = getenv("CLANE_NO_DIRECT") != nullptr;     // measurement aid
-    if (max_sweeps > 0 && max_sweeps <= 24 && !no_direct)
+    if (max_sweeps > 0 && max_sweeps <= 24)
         rc = clane_internal_sweeps_direct(s->plan, s->X, s->Z, start, s->rowptr, s->col, s->w, gamma, max_sweeps, s->state, s->log,
                                           s->log_cap, s->stream);
     else

@@ -8,8 +8,6 @@
 //   embedder.py:98-108 patience               -> patience_step (cascade.cuh)
 #include <math_constants.h>
 
-#include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <vector>
 #include <algorithm>
@@ -120,152 +118,6 @@ k_dots(const float* __restrict__ Za, const float* __restrict__ Zb, int ld, int d
         }
         if (lane < cnt) dots[e0 + lane] = acc;
     }
-}
-
-// ------------------------------------------------------------------------------------------
-// Dots AND the level-0 partials of the two global norms from ONE set of gathers (d in {32, 64, 128}: a row is whole cascade rows,
-// and a level-0 chunk of the cascade over [E*d] is `chunk_edges` = step * 32 / d whole edges, a power of two <= 32).
-// The norm cascade's lane m adds Z[row][32 s + m]^2 over the chunk's edges in order, s = 0..d/32-1 inside an edge: the two
-// rows of a round of 8 edges are parked once more in a small staging tile (lane = float4 of columns when written, lane =
-// cascade lane when read: conflict-free both ways), and every lane accumulates its cascade lane.  One 32-lane partial
-// per (chunk, norm) goes to P0n[chunk][2][32]; the last, incomplete chunk's partial is the cascade's "leftover rows".
-// Without this the norm cascade gathers the same 2 * E rows a second time (k_cascade_l01<ElemGatherSq2>: the two
-// kernels are L2-bandwidth-bound on 1.2 GB each at arxiv shape).
-// ------------------------------------------------------------------------------------------
-constexpr int kDotNormWarps = 4;
-constexpr size_t kDotNormWarpFloats = (size_t)32 * kDotPitch + 2 * 8 * kDotPitch;
-constexpr size_t kDotNormSmem = kDotNormWarps * kDotNormWarpFloats * sizeof(float);
-
-// the two rows of the 8 edges of round `i` of a tile: independent 128-bit loads (a source row equal to the previous edge's
-// is not loaded again: CSR order -- resolve_round copies it once the loads have landed)
-__device__ __forceinline__ void load_round(const float4* __restrict__ zc, int ra, int rb, int i, int prev_o, float4 (&x)[8],
-                                           float4 (&y)[8], int (&oa)[8]) {
-#pragma unroll
-    for (int u = 0; u < 8; ++u) {
-        oa[u] = __shfl_sync(kFull, ra, (i + u) & 31);
-        const int ob = __shfl_sync(kFull, rb, (i + u) & 31);
-        y[u] = __ldg(zc + ob);
-        if (oa[u] != (u == 0 ? prev_o : oa[u - 1])) x[u] = __ldg(zc + oa[u]);     // uniform branch
-    }
-}
-__device__ __forceinline__ void resolve_round(int prev_o, const float4& xprev, float4 (&x)[8], const int (&oa)[8]) {
-#pragma unroll
-    for (int u = 0; u < 8; ++u)
-        if (oa[u] == (u == 0 ? prev_o : oa[u - 1])) x[u] = u == 0 ? xprev : x[u - 1];
-}
-
-__global__ void __launch_bounds__(32 * kDotNormWarps)
-k_dots_norms(const float* __restrict__ Z, int ld, int d, const int32_t* __restrict__ erow, const int32_t* __restrict__ col,
-             int64_t E, int chunk_shift, float* __restrict__ dots, float* __restrict__ P0n) {
-    extern __shared__ __align__(16) float dot_tile[];
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    float* ta = dot_tile + (size_t)warp * kDotNormWarpFloats;     // products of 32 edges
-    float* sa = ta + 32 * kDotPitch;                              // source rows of a round of 8 edges
-    float* sb = sa + 8 * kDotPitch;                               // destination rows
-    const int64_t ntiles = (E + 31) / 32;
-    const int nseg = d >> 5;
-    const int64_t cmask = ((int64_t)1 << chunk_shift) - 1;
-    const int c = 4 * lane;
-    const bool in = c < ld;
-    const float4* zc = reinterpret_cast<const float4*>(Z) + (in ? c >> 2 : 0);
-    for (int64_t tile = (int64_t)blockIdx.x * kDotNormWarps + warp; tile < ntiles; tile += (int64_t)gridDim.x * kDotNormWarps) {
-        const int64_t e0 = tile * 32;
-        const int cnt = (int)min((int64_t)32, E - e0);
-        int ra = 0, rb = 0;
-        if (lane < cnt) { ra = __ldg(erow + e0 + lane) * (ld >> 2); rb = __ldg(col + e0 + lane) * (ld >> 2); }
-        int prev = -1;
-        float4 xprev = make_float4(0.f, 0.f, 0.f, 0.f);
-        float na = 0.0f, nb = 0.0f;                               // this lane's cascade lane of the open chunk
-        // two register buffers: the loads of round r + 1 are in flight while round r is parked and accumulated
-        float4 x[2][8], y[2][8];
-        int oa[2][8];
-        load_round(zc, ra, rb, 0, -1, x[0], y[0], oa[0]);
-#pragma unroll
-        for (int r = 0; r < 4; ++r) {
-            const int i = r * 8, b = r & 1;
-            if (i < cnt) {                                        // uniform
-                if (r < 3 && i + 8 < cnt) load_round(zc, ra, rb, i + 8, oa[b][7], x[b ^ 1], y[b ^ 1], oa[b ^ 1]);
-                resolve_round(prev, xprev, x[b], oa[b]);
-                prev = oa[b][7];
-                xprev = x[b][7];
-                __syncwarp();                                     // the previous round's staging has been read
-#pragma unroll
-                for (int u = 0; u < 8; ++u) {
-                    *reinterpret_cast<float4*>(ta + (i + u) * kDotPitch + c) =
-                        make_float4(fmul(x[b][u].x, y[b][u].x), fmul(x[b][u].y, y[b][u].y), fmul(x[b][u].z, y[b][u].z),
-                                    fmul(x[b][u].w, y[b][u].w));
-                    *reinterpret_cast<float4*>(sa + u * kDotPitch + c) = x[b][u];
-                    *reinterpret_cast<float4*>(sb + u * kDotPitch + c) = y[b][u];
-                }
-                __syncwarp();
-                // all of the round's squares first (independent shared-memory reads), then the two in-order chains
-                float qa[8][4], qb[8][4];
-#pragma unroll
-                for (int u = 0; u < 8; ++u)
-#pragma unroll
-                    for (int sg = 0; sg < 4; ++sg) {
-                        const float xa = sg < nseg ? sa[u * kDotPitch + 32 * sg + lane] : 0.0f;
-                        const float xb = sg < nseg ? sb[u * kDotPitch + 32 * sg + lane] : 0.0f;
-                        qa[u][sg] = fmul(xa, xa);
-                        qb[u][sg] = fmul(xb, xb);
-                    }
-#pragma unroll
-                for (int u = 0; u < 8; ++u) {
-                    if (i + u < cnt) {                            // uniform
-                        const int64_t e = e0 + i + u;
-                        if ((e & cmask) == 0) { na = 0.0f; nb = 0.0f; }   // a chunk opens
-#pragma unroll
-                        for (int sg = 0; sg < 4; ++sg)
-                            if (sg < nseg) {
-                                na = fadd(na, qa[u][sg]);
-                                nb = fadd(nb, qb[u][sg]);
-                            }
-                        if (((e + 1) & cmask) == 0 || e + 1 == E) {   // the chunk closes (or the array ends inside it)
-                            float* o = P0n + (size_t)(e >> chunk_shift) * 64 + lane;
-                            o[0] = na;
-                            o[32] = nb;
-                        }
-                    }
-                }
-            }
-        }
-        __syncwarp();
-        // lane i sums edge i in feature order
-        const float* pp = ta + lane * kDotPitch;
-        float acc = 0.0f;
-        for (int j = 0; j < d; j += 4) {
-            const float4 q = *reinterpret_cast<const float4*>(pp + j);
-            acc = fadd(acc, q.x); acc = fadd(acc, q.y); acc = fadd(acc, q.z); acc = fadd(acc, q.w);
-        }
-        if (lane < cnt) dots[e0 + lane] = acc;
-        __syncwarp();
-    }
-}
-
-// level 1 of the two norms from the chunk partials of k_dots_norms: `step` consecutive chunks per node, in order
-__global__ void __launch_bounds__(256)
-k_level1_from_p0n(CascadeShape sh, const float* __restrict__ P0n, float* __restrict__ ws) {
-    const int lane = threadIdx.x & 31;
-    const int64_t w = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;     // (node, norm)
-    const int64_t node = w >> 1;
-    const int q = (int)(w & 1);
-    if (node >= sh.n1_nodes) return;
-    const int step = (int)sh.step;
-    const int cnt = node < sh.n1_full ? step : (int)sh.c_rem;
-    const float* src = P0n + ((size_t)node * step * 2 + q) * 32 + lane;
-    float acc = 0.0f;
-    int i = 0;
-    for (; i + 8 <= cnt; i += 8) {
-        float v[8];
-#pragma unroll
-        for (int u = 0; u < 8; ++u) v[u] = __ldg(src + (size_t)(i + u) * 64);
-#pragma unroll
-        for (int u = 0; u < 8; ++u) acc = fadd(acc, v[u]);
-    }
-    for (; i < cnt; ++i) acc = fadd(acc, __ldg(src + (size_t)i * 64));
-    ws[((size_t)node * 2 + q) * 32 + lane] = acc;
-    if (node == sh.n1_nodes - 1 && sh.rem_rows > 0 && sh.r_rem > 0)               // leftover rows = the last, partial chunk
-        ws[(size_t)(sh.n1_nodes + 1) * 64 + q * 32 + lane] = __ldg(P0n + ((size_t)(sh.n1_full * step + sh.c_rem) * 2 + q) * 32 + lane);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -448,35 +300,14 @@ namespace {
 
 // kernel launch with an explicit priority: the attribute stays on the kernel node when the launch is captured into a
 // graph (a captured node does not reliably inherit the priority of the stream it was captured from)
-// measurement aid (CLANE_L2_WINDOW): an L2 access-policy window the next launch carries
-thread_local const cudaAccessPolicyWindow* tl_window = nullptr;
-// sets the persisting share of the L2 aside once (not allowed while a stream captures: called before); the largest window
-int l2_window_max() {
-    static int max_win = -1;
-    if (max_win < 0) {
-        int dev = 0, max_persist = 0;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&max_persist, cudaDevAttrMaxPersistingL2CacheSize, dev);
-        cudaDeviceGetAttribute(&max_win, cudaDevAttrMaxAccessPolicyWindowSize, dev);
-        cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, (size_t)max_persist);
-        fprintf(stderr, "clane: L2 window: max persisting %d MB, max window %d MB\n", max_persist >> 20, max_win >> 20);
-    }
-    return max_win;
-}
 template <class... KArgs, class... Args>
 cudaError_t launch_prio(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, int prio, Args... args) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
-    cudaLaunchAttribute attr[2];
-    attr[0].id = cudaLaunchAttributePriority;
-    attr[0].val.priority = prio;
-    cfg.attrs = attr; cfg.numAttrs = 1;
-    if (tl_window != nullptr) {
-        attr[1].id = cudaLaunchAttributeAccessPolicyWindow;
-        attr[1].val.accessPolicyWindow = *tl_window;
-        cfg.numAttrs = 2;
-        tl_window = nullptr;
-    }
+    cudaLaunchAttribute attr;
+    attr.id = cudaLaunchAttributePriority;
+    attr.val.priority = prio;
+    cfg.attrs = &attr; cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
 }
 
@@ -485,8 +316,9 @@ cudaError_t launch_prio(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t 
 using namespace clane;
 
 constexpr int kSweepBatch = 6;     // sweeps per replayed graph of clane_sweeps (a multiple of the three Z buffers)
-constexpr int kWhileBatch = 6;     // sweeps per iteration of the conditional-WHILE body (until_stop); CLANE_WHILE_BATCH = 12 / 24
-                                   // measured no better (arxiv shape, time to converge 0.105 / 0.107 / 0.115 s)
+constexpr int kWhileBatch = 6;     // sweeps per iteration of the conditional-WHILE body (until_stop); 12 / 24 measured
+                                   // no better (arxiv shape, time to converge 0.105 / 0.107 / 0.115 s)
+static_assert(kSweepBatch % 3 == 0 && kWhileBatch % 3 == 0, "a batch returns the three Z buffers to where it started");
 // The L1 tail of sweep t runs while the span tasks of sweep t + 1 fill every SM (12 CTAs x 64 threads x 80 registers leave
 // 4096 registers per SM): 64-thread CTAs of <= 64 registers are what still fits beside them.
 constexpr int kTailThreads = 64;
@@ -548,39 +380,9 @@ int clane_scores_cosine(clane_plan* plan, const float* d_Z, const int32_t* d_ero
     if (!plan || !d_Z || !d_erow || !d_col || !d_dots) return CLANE_EINVAL;
     if (edge_lo < 0 || edge_hi > plan->e || edge_lo > edge_hi) return CLANE_EINVAL;
     cudaStream_t st = (cudaStream_t)s;
-    // One pass for the dots and the norms' level-0 partials when a chunk of the cascade is a few whole edges: OPT-IN
-    // (CLANE_FUSED_NORMS=1).  Measured at arxiv shape: build_P 0.336 ms against 0.304 ms for the two kernels side by side --
-    // the tile + staging leave 8 warps per SM, and the in-order chains of phases B and C then stall the issue slots
-    // (profiles/r02_notes.md).  Bit-exact either way (tests/test_gpu_parity.py::test_dots_and_norms_from_one_pass).
-    const char* fuse_env = getenv("CLANE_FUSED_NORMS");
-    if (d_norms2 != nullptr && edge_lo == 0 && edge_hi == plan->e && plan->e > 0 && fuse_env && atoi(fuse_env) != 0 &&
-        (plan->d == 32 || plan->d == 64 || plan->d == 128)) {
-        const CascadeShape sh = cascade_shape(plan->e * (int64_t)plan->d);
-        const int64_t chunk_edges = sh.step * 32 / plan->d;
-        if (chunk_edges >= 1 && chunk_edges <= 32) {
-            int shift = 0;
-            while (((int64_t)1 << shift) < chunk_edges) ++shift;
-            const size_t need = (size_t)((plan->e >> shift) + 1) * 64;
-            if (plan->p0n_floats < need) {
-                if (plan->d_p0n) CLANE_CUDA(cudaFree(plan->d_p0n));
-                plan->d_p0n = nullptr; plan->p0n_floats = 0;
-                CLANE_CUDA(cudaMalloc(&plan->d_p0n, need * sizeof(float)));
-                plan->p0n_floats = need;
-            }
-            const int64_t ntiles = (plan->e + 31) / 32;
-            const unsigned grid = (unsigned)std::min<int64_t>((ntiles + kDotNormWarps - 1) / kDotNormWarps, 148 * 16);
-            k_dots_norms<<<grid, 32 * kDotNormWarps, kDotNormSmem, st>>>(d_Z, plan->ld, plan->d, d_erow, d_col, plan->e, shift, d_dots,
-                                                                    plan->d_p0n);
-            CLANE_LAUNCH_CHECK();
-            const int64_t warps = sh.n1_nodes * 2;
-            k_level1_from_p0n<<<(unsigned)((warps * 32 + 255) / 256), 256, 0, st>>>(sh, plan->d_p0n, plan->d_p1);
-            CLANE_LAUNCH_CHECK();
-            ElemGatherSq2 el{d_Z, d_erow, d_col, plan->d, plan->ld, plan->e};
-            return cascade_launch_finish(el, plan->e * (int64_t)plan->d, plan->d_p1, plan->d_p2, d_norms2, nullptr, nullptr, 0, nullptr, st);
-        }
-    }
     // the dots and the norm cascade are independent and both latency-bound at partial occupancy: with a schedule plan (it
-    // owns side streams) the dots run on a side stream beside the cascade on the caller's
+    // owns side streams) the dots run on a side stream beside the cascade on the caller's.  (One kernel gathering once for
+    // both was measured slower at arxiv shape, 0.336 against 0.304 ms: profiles/r02_notes.md.)
     cudaStream_t caller = st;
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
     const bool beside = d_norms2 != nullptr && plan->side != nullptr && edge_hi > edge_lo;
@@ -774,7 +576,6 @@ static int enqueue_sweeps(clane_plan* plan, const SweepArgs& a, float* const* Z,
         cudaError_t rc = next_event(ev);
         return rc != cudaSuccess ? rc : cudaEventRecord(*ev, s);
     };
-    static const bool no_peer_stores = getenv("CLANE_DEBUG_NO_PEER_STORES") != nullptr;   // timing experiments only
     const int per_row = plan->nslab32b + (plan->ntail4 > 0 ? 1 : 0);
     const int n_long = plan->n_long_hub_rows, n_short = plan->n_hub_rows - n_long;
     const bool hubs = plan->n_hub_rows > 0 && plan->n_seg_tasks > 0;
@@ -810,15 +611,14 @@ static int enqueue_sweeps(clane_plan* plan, const SweepArgs& a, float* const* Z,
         p.bulk = 0;
         p.trace = nullptr;
         unsigned long long* tr = (plan->d_trace != nullptr && t < kTraceSweeps) ? plan->d_trace + (size_t)t * kTraceSlots * 2 : nullptr;
-        for (int q = 0; q < 3 && plan->n_peers > 1 && !no_peer_stores; ++q)
+        for (int q = 0; q < 3 && plan->n_peers > 1; ++q)
             if (plan->peers[q][plan->self_rank] == Zn) {
                 if (plan->mc[q] != nullptr) { p.mc = plan->mc[q]; continue; }   // one multicast store instead of n - 1 unicast ones
                 for (int r = 0; r < plan->n_peers; ++r)
                     if (r != plan->self_rank) p.peer[p.n_remote++] = plan->peers[q][r];
             }
         // whole rows per warp and unicast peers: the spans' rows leave as bulk stores (sweep.cuh, flush_rows)
-        static const char* bulk_env = getenv("CLANE_PEER_BULK");         // 0: lane stores (measurement aid)
-        if (p.n_remote > 0 && plan->nslab == 1 && plan->G <= kStageRows && !(bulk_env && atoi(bulk_env) == 0)) p.bulk = 1;
+        if (p.n_remote > 0 && plan->nslab == 1 && plan->G <= kStageRows) p.bulk = 1;
         // what the previous sweeps must have finished before this one may start
         cudaEvent_t prev_tail = nullptr;       // the tail whose inputs this sweep overwrites / whose flag it reads
         if (nz >= 3) { if (t >= 2) prev_tail = eL[t - 2]; }
@@ -864,25 +664,12 @@ static int enqueue_sweeps(clane_plan* plan, const SweepArgs& a, float* const* Z,
         // The segments and the light chains fit beside the span CTAs (sweep.cuh), so normally the spans do not wait for
         // them.  Heavy chains want an SM each: with long hub rows the spans start behind the segments, together with the
         // heavy chains, which the higher priority places first (the segments are microseconds of a millisecond sweep).
-        static const char* seg_wait_env = getenv("CLANE_SEG_WAIT");     // 0 / 1: measurement aid
-        const bool seg_wait = seg_wait_env ? atoi(seg_wait_env) != 0 : n_long > 0;
-        if (eS_cur && seg_wait) CLANE_CUDA(cudaStreamWaitEvent(st, eS_cur, 0));
+        if (eS_cur && n_long > 0) CLANE_CUDA(cudaStreamWaitEvent(st, eS_cur, 0));
         if (prof) CLANE_CUDA(prof_mark(plan, 1, st));
         if (span_ctas > 0) {
             SweepParams pr = p;
             pr.task_lo = plan->n_seg_tasks;
             pr.trace = tr ? tr + 6 : nullptr;
-            static const char* win_env = getenv("CLANE_L2_WINDOW");     // hit ratio of a persisting window over Zcur
-            cudaAccessPolicyWindow win = {};
-            if (win_env && atof(win_env) > 0.0) {
-                int max_win = l2_window_max();
-                win.base_ptr = const_cast<float*>(Zc);
-                win.num_bytes = std::min<size_t>((size_t)plan->n * plan->ld * 4, (size_t)max_win);
-                win.hitRatio = (float)atof(win_env);
-                win.hitProp = cudaAccessPropertyPersisting;
-                win.missProp = cudaAccessPropertyNormal;
-                tl_window = &win;
-            }
             if (pr.bulk)
                 CLANE_CUDA(launch_prio(k_sweep_rows<true>, dim3((unsigned)span_ctas), dim3(kRowThreads), kRowWarps * kRowStageBytes, st,
                                        plan->prio_lo, pr));
@@ -943,17 +730,13 @@ static int enqueue_sweeps(clane_plan* plan, const SweepArgs& a, float* const* Z,
 // body of a conditional WHILE node that repeats it until the patience state machine stops (one launch = one propagate()).
 static int launch_sweeps(clane_plan* plan, const SweepArgs& a, float* const* Z, int nz, int c0, int n_sweeps, int loop,
                          cudaStream_t st) {
-    static const bool env_graphs = getenv("CLANE_NO_GRAPHS") == nullptr;
     cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
     cudaStreamIsCapturing(st, &cap);
-    static const bool env_force = getenv("CLANE_FORCE_GRAPHS") != nullptr;   // measurement aid
-    if (!plan->use_graphs || !env_graphs || cap != cudaStreamCaptureStatusNone || st == nullptr ||
-        (plan->prefer_direct && !env_force)) {
+    if (!plan->use_graphs || cap != cudaStreamCaptureStatusNone || st == nullptr) {
         if (loop) return CLANE_EINVAL;   // the caller falls back to host-driven batches
         return enqueue_sweeps(plan, a, Z, nz, c0, n_sweeps, st);
     }
     const void* key[12] = {a.X, Z[0], Z[1], nz > 2 ? Z[2] : nullptr, a.rowptr, a.col, a.w, a.amount, a.state, a.log, st, nullptr};
-    if (getenv("CLANE_L2_WINDOW")) l2_window_max();
     clane_plan::SweepGraph* slot = nullptr;
     for (auto& g : plan->graphs)
         if (g.exec && g.gamma == a.gamma && g.log_cap == a.log_cap && g.n_sweeps == n_sweeps && g.nz == nz && g.c0 == c0 &&
@@ -1058,24 +841,17 @@ int clane_sweeps(clane_plan* plan, const float* d_X, float* const* d_Z3, int32_t
     if (rc != CLANE_OK) return rc;
     SweepArgs a{d_X, d_rowptr, d_col, d_w, gamma, nullptr, d_state, d_amounts_log, log_cap};
     if (until_stop) {
-        static const bool env_force = getenv("CLANE_FORCE_GRAPHS") != nullptr;
-        if (!plan->while_ok || (plan->prefer_direct && !env_force)) return CLANE_EUNSUPPORTED;
-        // sweeps per iteration of the WHILE body (a multiple of 3: the body always starts at buffer `cur`)
-        static const int body = [] {
-            const char* v = getenv("CLANE_WHILE_BATCH");
-            const int b = v ? atoi(v) : kWhileBatch;
-            return std::max(3, b - b % 3);
-        }();
-        rc = launch_sweeps(plan, a, d_Z3, 3, cur, body, 1, st);
+        if (!plan->while_ok) return CLANE_EUNSUPPORTED;
+        // the WHILE body always starts at buffer `cur` (kWhileBatch is a multiple of 3)
+        rc = launch_sweeps(plan, a, d_Z3, 3, cur, kWhileBatch, 1, st);
         return rc == CLANE_EINVAL ? CLANE_EUNSUPPORTED : rc;
     }
     // whole batches replay one cached graph per starting buffer (kSweepBatch is a multiple of 3: the rotation closes)
-    static const int batch = [] { const char* v = getenv("CLANE_SWEEP_BATCH"); return v ? std::max(1, atoi(v)) : kSweepBatch; }();
     int done = 0;
-    while (n_sweeps - done >= batch) {
-        rc = launch_sweeps(plan, a, d_Z3, 3, (cur + done) % 3, batch, 0, st);
+    while (n_sweeps - done >= kSweepBatch) {
+        rc = launch_sweeps(plan, a, d_Z3, 3, (cur + done) % 3, kSweepBatch, 0, st);
         if (rc != CLANE_OK) return rc;
-        done += batch;
+        done += kSweepBatch;
     }
     if (n_sweeps > done) rc = launch_sweeps(plan, a, d_Z3, 3, (cur + done) % 3, n_sweeps - done, 0, st);
     return rc;
@@ -1230,9 +1006,6 @@ int clane_internal_prepare_kernels(void) {
     CLANE_CUDA(cudaFuncSetAttribute(k_hub_chain<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kHeavySmemBytes));
     CLANE_CUDA(cudaFuncSetAttribute(k_dots<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dot_smem<false>()));
     CLANE_CUDA(cudaFuncSetAttribute(k_dots<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dot_smem<true>()));
-    CLANE_CUDA(cudaFuncSetAttribute(k_dots_norms, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kDotNormSmem));
-    if (const char* v = getenv("CLANE_ROW_CARVEOUT"))    // timing experiments: shared-memory carveout (percent) of the row kernel
-        CLANE_CUDA(cudaFuncSetAttribute(k_sweep_rows<false>, cudaFuncAttributePreferredSharedMemoryCarveout, atoi(v)));
     // the cascade level-0/1 kernel needs step*NQ*128 bytes (<= 32 KB for step = 128, NQ = 2)
     done = true;
     return CLANE_OK;

@@ -53,7 +53,6 @@ struct clane_plan {
     } graphs[6];
     unsigned long long graph_clock = 0;
     bool use_graphs = true;
-    bool prefer_direct = false;        // enqueue sweeps directly instead of replaying graphs (CLANE_PREFER_DIRECT: measurement aid)
     bool while_ok = true;              // conditional-WHILE graphs available (cleared when their creation fails once)
     bool profile = false;              // record timing events around the kernels of each sweep
     cudaEvent_t ev_prof[8] = {};
@@ -64,8 +63,6 @@ struct clane_plan {
     // cascade scratch: level-1 slots and level-2 slots, sized for max(n*d x1, e*d x2)
     float* d_p1 = nullptr;
     float* d_p2 = nullptr;
-    float* d_p0n = nullptr;     // build_P: level-0 partials of the two norms from k_dots_norms, [chunk][2][32] (allocated on first use)
-    size_t p0n_floats = 0;
     size_t p1_floats = 0, p2_floats = 0;
 };
 

@@ -2,11 +2,6 @@
 #pragma once
 #include <stdint.h>
 
-// resident warps per SM the row kernel is compiled for (register budget: 65536 / (32 * warps) per thread)
-#ifndef CLANE_ROW_WARPS_PER_SM
-#define CLANE_ROW_WARPS_PER_SM 24
-#endif
-
 namespace clane {
 
 // One warp's work: a span (consecutive ordinary rows of one row group) or a hub segment.  Two int4; a span only

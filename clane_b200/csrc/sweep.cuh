@@ -33,10 +33,6 @@
 #include "common.cuh"
 #include "program.cuh"
 
-#ifndef CLANE_DEBUG_GATHER_MASK       // timing experiments only: fold every gather into a small table (wrong results)
-#define CLANE_DEBUG_GATHER_MASK 0xffffffffu
-#endif
-
 namespace clane {
 
 struct SweepParams {
@@ -93,12 +89,10 @@ __global__ void k_trace_stamp(unsigned long long* tr, int end) {
     if (end) atomicMax(tr + 1, globaltimer_ns()); else atomicMin(tr, globaltimer_ns());
 }
 
-#ifndef CLANE_ROW_WARPS
-#define CLANE_ROW_WARPS 2
-#endif
-constexpr int kRowWarps = CLANE_ROW_WARPS;     // row kernel: warps (= tasks) per CTA
+constexpr int kRowWarps = 2;                   // row kernel: warps (= tasks) per CTA
 constexpr int kRowThreads = 32 * kRowWarps;
-constexpr int kRowWarpsPerSM = CLANE_ROW_WARPS_PER_SM;   // the register budget the row kernel is compiled for
+// resident warps per SM the row kernel is compiled for (register budget: 65536 / (32 * warps) per thread)
+constexpr int kRowWarpsPerSM = 24;
 // row kernel shared memory per warp: (offset, w) window | two 512-byte transpose buffers (fused L1) | the row's X and
 // own Zcur pieces (cp.async) | stream position of a row longer than the window
 constexpr size_t kRowWarpSmem = (size_t)kMetaRing * sizeof(int2) + 2 * 512 + 2 * 512 + 16;
@@ -225,15 +219,9 @@ __device__ __forceinline__ void ldg_f32_if(float& v, const float* p, bool pred) 
 // sector hit rate stays at 44 % either way and the policy descriptors cost 8 % more instructions (R2UR / UMOV),
 // so plain accesses are used; Znext is written with the streaming (.cs) qualifier.
 // neighbour row piece of this lane: 16 bytes at float4 index `off16` of the lane's column base
+// (an unsigned index: the address is a 32-bit unsigned multiply-add, IMAD.WIDE.U32)
 __device__ __forceinline__ float4 gather4(const float4* __restrict__ zb, int off16) {
-#ifdef CLANE_GATHER_NO_L1
-    float4 v;
-    asm volatile("ld.global.nc.L1::no_allocate.v4.f32 {%0, %1, %2, %3}, [%4];"
-                 : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(zb + ((unsigned)off16 & CLANE_DEBUG_GATHER_MASK)));
-    return v;
-#else
-    return __ldg(zb + ((unsigned)off16 & CLANE_DEBUG_GATHER_MASK));
-#endif
+    return __ldg(zb + (unsigned)off16);
 }
 __device__ __forceinline__ float4 ldg_stream4(const float* p) {   // X: read once per sweep, keep it out of L1
     float4 v;
@@ -315,27 +303,6 @@ __device__ __forceinline__ void flush_rows(const SweepParams& p, const float* st
         bulk_commit();
     }
 }
-#ifndef CLANE_PF_AHEAD
-#define CLANE_PF_AHEAD 0       // window positions the L2 prefetch of neighbour rows runs ahead of the gathers (0: off)
-#endif
-#ifndef CLANE_PF_XOWN
-#define CLANE_PF_XOWN 1        // request the span's X / own Zcur lines when the span opens
-#endif
-// L2 prefetch of the neighbour rows of window entries [pf, pf + 8): lane L takes line L % 4 of entry pf + L / 4, so
-// one instruction covers the 8 x 512 bytes of a whole batch.  The kernel is bound by the latency of its gathers
-// (a batch waits for the slowest of <= 8 rows, and half of them miss the L2): a row requested one or two batches
-// early turns that DRAM round trip into an L2 hit.  No register, no scoreboard: fire and forget.
-__device__ __forceinline__ void prefetch_batch(const float* zslab, int slab_bytes, const int2* meta, int pf, int cnt, int lane) {
-    const int i = pf + (lane >> 2), line = (lane & 3) * 128;
-    if (i < cnt && line < slab_bytes) {
-        const char* a = reinterpret_cast<const char*>(zslab) + (size_t)((unsigned)meta[i].x & CLANE_DEBUG_GATHER_MASK) * 16 + line;
-#ifdef CLANE_PF_L1
-        asm volatile("prefetch.global.L1 [%0];" ::"l"(a));
-#else
-        prefetch_l2(a);
-#endif
-    }
-}
 
 // (offset, w) pairs of up to kMetaRing consecutive edges of the task's stream, starting at edge `e0` (cnt left)
 // -> the warp's shared-memory window.  Four predicated, independent load pairs per lane: one round trip.
@@ -395,24 +362,18 @@ __device__ __forceinline__ void run_span(const SweepParams& p, const int4 t0, in
     const int nseg = p.d >> 5;
     int mpos = 0;                              // position inside the window
     float chunk_acc = 0.0f;
-    const float* zslab = p.Zc + slab * 128;
     const int slab_bytes = min(128, p.ld - slab * 128) * 4;
-    int wcnt = min(t0.y, kMetaRing), pf = 0;   // entries in the window; entries whose rows are already requested
-    if (CLANE_PF_XOWN) {
-        // the rows' X and own Zcur pieces, known in advance: request the span's lines now
-        if (p.nslab == 1) {                    // consecutive rows are contiguous: one line per lane
-            const int bytes = nrows * p.ld * 4, o = lane * 128;
-            if (o < bytes) {
-                prefetch_l2(reinterpret_cast<const char*>(p.X + (size_t)r0 * p.ld) + o);
-                if (direct) prefetch_l2(reinterpret_cast<const char*>(p.Zc + (size_t)r0 * p.ld) + o);
-            }
-        } else if ((lane >> 2) < nrows && (lane & 3) * 128 < slab_bytes) {
-            const size_t o = ((size_t)(r0 + (lane >> 2)) * p.ld + slab * 128) * 4 + (lane & 3) * 128;
-            prefetch_l2(reinterpret_cast<const char*>(p.X) + o);
+    // the rows' X and own Zcur pieces, known in advance: request the span's lines now
+    if (p.nslab == 1) {                        // consecutive rows are contiguous: one line per lane
+        const int bytes = nrows * p.ld * 4, o = lane * 128;
+        if (o < bytes) {
+            prefetch_l2(reinterpret_cast<const char*>(p.X + (size_t)r0 * p.ld) + o);
+            if (direct) prefetch_l2(reinterpret_cast<const char*>(p.Zc + (size_t)r0 * p.ld) + o);
         }
+    } else if ((lane >> 2) < nrows && (lane & 3) * 128 < slab_bytes) {
+        const size_t o = ((size_t)(r0 + (lane >> 2)) * p.ld + slab * 128) * 4 + (lane & 3) * 128;
+        prefetch_l2(reinterpret_cast<const char*>(p.X) + o);
     }
-    if (CLANE_PF_AHEAD > 0)
-        for (; pf < CLANE_PF_AHEAD && pf < wcnt; pf += 8) prefetch_batch(zslab, slab_bytes, meta, pf, wcnt, lane);
     int run0 = -1;                             // bulk mode: first row of the run of finished rows parked in `stage`
     for (int r = 0; r < nrows; ++r) {
         int k = __shfl_sync(kFull, deg, r);
@@ -420,32 +381,18 @@ __device__ __forceinline__ void run_span(const SweepParams& p, const int4 t0, in
             if (kBulk && run0 >= 0) { flush_rows(p, stage, r0, run0, r, lane); run0 = -1; }
             continue;
         }
-        {
-#ifdef CLANE_DEBUG_ROW0          // timing experiments only: every row's X / own / Znext piece is row 0's (wrong results)
-            const int row_off = cc;
-#else
-            const int row_off = (r0 + r) * p.ld + cc;      // n * ld < 2^31 (clane_plan_create)
-#endif
-            cp_async16_sa(rowbuf_sa, p.X + row_off);
-            if (direct) cp_async16_sa(rowbuf_sa + 512, p.Zc + row_off);
-            cp_async_commit();
-        }
+        const int row_off = (r0 + r) * p.ld + cc;          // n * ld < 2^31 (clane_plan_create)
+        cp_async16_sa(rowbuf_sa, p.X + row_off);
+        if (direct) cp_async16_sa(rowbuf_sa + 512, p.Zc + row_off);
+        cp_async_commit();
         float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
         for (; k >= 8; k -= 8) {
-            if (mpos == kMetaRing) { restage_meta(p, lane, meta, state); mpos = 0; pf = 0; wcnt = min(state[1], kMetaRing); }
-            if (CLANE_PF_AHEAD > 0 && pf < wcnt && pf < mpos + 8 + CLANE_PF_AHEAD) {
-                prefetch_batch(zslab, slab_bytes, meta, pf, wcnt, lane);
-                pf += 8;
-            }
+            if (mpos == kMetaRing) { restage_meta(p, lane, meta, state); mpos = 0; }
             block_batch(meta + mpos, zb, acc, all_blocked, col_blocked);
             mpos += 8;
         }
         if (k != 0) {
-            if (mpos == kMetaRing) { restage_meta(p, lane, meta, state); mpos = 0; pf = 0; wcnt = min(state[1], kMetaRing); }
-            if (CLANE_PF_AHEAD > 0 && pf < wcnt && pf < mpos + 8 + CLANE_PF_AHEAD) {
-                prefetch_batch(zslab, slab_bytes, meta, pf, wcnt, lane);
-                pf += 8;
-            }
+            if (mpos == kMetaRing) { restage_meta(p, lane, meta, state); mpos = 0; }
             const int2* mp = meta + mpos;
             switch (k) {
                 case 1: seq_batch<1>(mp, zb, acc); break;
@@ -460,11 +407,6 @@ __device__ __forceinline__ void run_span(const SweepParams& p, const int4 t0, in
         }
         cp_async_wait<0>();                    // each lane reads back the 16 bytes it copied itself: no barrier
         const float4 out = finish_row(rowbuf[lane], acc, p.gamma);
-#ifdef CLANE_DEBUG_ROW0
-        const int row_off = cc;
-#else
-        const int row_off = (r0 + r) * p.ld + cc;
-#endif
         if (kBulk) {
             if (active) *reinterpret_cast<float4*>(stage + r * p.ld + cc) = out;
             if (run0 < 0) run0 = r;

@@ -7,7 +7,6 @@ reproduce the reference's rounding sequence, every comparison below is also asse
 BIT-EXACT (np.array_equal), which implies the stated tolerance.
 """
 import ctypes
-import os
 from pathlib import Path
 
 import numpy as np
@@ -444,9 +443,8 @@ def test_adjacent_hub_rows_across_build_p_calls(monkeypatch):
 
 
 def while_launch_required() -> bool:
-    """clane_sweeps(until_stop=1) must take the conditional-WHILE graph on a B200 unless graphs are switched off."""
-    return (torch.cuda.get_device_capability()[0] == 10 and not os.environ.get("CLANE_PREFER_DIRECT")
-            and not os.environ.get("CLANE_NO_GRAPHS"))
+    """clane_sweeps(until_stop=1) must take the conditional-WHILE graph on a B200."""
+    return torch.cuda.get_device_capability()[0] == 10
 
 
 def test_sweeps_batches_equal_single_sweeps():
@@ -533,11 +531,10 @@ def test_norms_reduced_by_node_range_equal_whole():
 
 @pytest.mark.parametrize("n,e,d", [(50, 3, 128), (50, 33, 128), (900, 4001, 128), (40000, 270003, 128), (700, 3001, 64),
                                    (30000, 530001, 64), (900, 5003, 32), (60000, 1050007, 32)])
-def test_dots_and_norms_from_one_pass(n, e, d, monkeypatch):
-    """k_dots_norms (opt-in, CLANE_FUSED_NORMS=1; d = 32 / 64 / 128: the norms' level-0 partials come from the gathers
-    of the dots) against the oracle and against the default two-kernel form, at every chunk size (4 / 8 / 16 / 32 edges
-    per level-0 chunk), with partial last chunks and partial tiles."""
-    monkeypatch.setenv("CLANE_FUSED_NORMS", "1")
+def test_scores_cosine_every_norm_chunk_size(n, e, d):
+    """clane_scores_cosine (the dots on a side stream beside the norm cascade) against the oracle at every level-0
+    chunk size of the norm cascade (4 / 8 / 16 / 32 edges per chunk at d = 128 / 64 / 32), with partial last chunks
+    and partial tiles of 32 edges."""
     L = _lib.lib()
     rng = np.random.default_rng(n + e + d)
     src, dst = synth.make_edges(n, e, "powerlaw" if n >= 900 else "uniform", rng)
@@ -555,11 +552,6 @@ def test_dots_and_norms_from_one_pass(n, e, d, monkeypatch):
     od, s1, s2 = O.scores_raw(X, rowptr, col)
     assert np.array_equal(dots.cpu().numpy(), od)
     assert norms.cpu().numpy().tolist() == [s1, s2]
-    monkeypatch.setenv("CLANE_FUSED_NORMS", "0")
-    dots2, norms2 = torch.zeros_like(dots), torch.zeros_like(norms)
-    _lib.check(L.clane_scores_cosine(S.plan.handle, S.Z[0].data_ptr(), S.erow.data_ptr(), S.col.data_ptr(), 0, S.e,
-                                     dots2.data_ptr(), norms2.data_ptr(), s))
-    assert torch.equal(dots, dots2) and torch.equal(norms, norms2)
 
 
 @pytest.mark.parametrize("n,d", [(1000, 128), (300, 64), (4097, 32), (777, 96)])
