@@ -67,6 +67,9 @@ SIGNATURES = {
     "clane_asym_supported": (C.c_int, [C.c_int32]),
     "clane_asym_project": (C.c_int, [c_vp, C.c_int32, C.c_int32, C.c_int32, c_vp, c_vp, c_vp, c_vp, c_vp]),
     "clane_build_p_asym": (C.c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    "clane_asym_project_fp32": (C.c_int, [c_vp, C.c_int32, C.c_int32, C.c_int32, c_vp, C.c_int32, c_vp, c_vp, c_vp, c_vp,
+                                          c_vp]),
+    "clane_build_p_asym_fp32": (C.c_int, [c_vp, c_vp, c_vp, C.c_int32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
     "clane_cosine_finalize": (C.c_int, [c_vp, c_vp, C.c_int64, c_vp, c_vp]),
     "clane_build_p_cosine": (C.c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
     "clane_sweep": (C.c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, C.c_float, c_vp, c_vp, c_vp, C.c_int32, c_vp]),

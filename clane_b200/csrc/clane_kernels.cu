@@ -495,6 +495,34 @@ int clane_build_p_asym(clane_plan* plan, const float* d_Z, const float* d_W, con
     return clane_plan_softmax(plan, d_w, nullptr, d_rowptr, d_w, s);     // graph.py:122-123: no norm divisor for this plugin
 }
 
+int clane_build_p_asym_fp32(clane_plan* plan, const float* d_Z, const float* d_W, int32_t ldw, const int32_t* d_rowptr,
+                            const int32_t* d_erow, const int32_t* d_col, float* d_w, float* d_work, int32_t* d_error,
+                            clane_stream_t s) {
+    if (!plan || !plan->has_schedule || !d_Z || !d_W || !d_rowptr || !d_w || !d_work || !d_error) return CLANE_EINVAL;
+    if (plan->e > 0 && (!d_erow || !d_col)) return CLANE_EINVAL;
+    float* psrc = d_work;
+    float* pdst = d_work + (size_t)plan->n * plan->ld;
+    // every node projected once, 3xTF32 on the tensor cores; the weight split goes after the two projected matrices
+    int rc = clane_asym_project_fp32(d_Z, plan->n, plan->d, plan->ld, d_W, ldw, psrc, pdst, pdst + (size_t)plan->n * plan->ld,
+                                     d_error, s);
+    if (rc != CLANE_OK) return rc;
+    const int64_t e_lo = plan->edge_lo, e_hi = plan->edge_hi;
+    if (e_hi > e_lo) {
+        // the reference's bmm: mul + add below d = 400, fma from there on (as the cosine path)
+        const int64_t ntiles = (e_hi - e_lo + 31) / 32;
+        cudaStream_t st = (cudaStream_t)s;
+        if (plan->d < 400) {
+            const unsigned grid = (unsigned)std::min<int64_t>((ntiles + dot_warps<false>() - 1) / dot_warps<false>(), 148 * 24);
+            k_dots<false><<<grid, 32 * dot_warps<false>(), dot_smem<false>(), st>>>(psrc, pdst, plan->ld, plan->d, d_erow, d_col, e_lo, e_hi, d_w);
+        } else {
+            const unsigned grid = (unsigned)std::min<int64_t>((ntiles + dot_warps<true>() - 1) / dot_warps<true>(), 148 * 24);
+            k_dots<true><<<grid, 32 * dot_warps<true>(), dot_smem<true>(), st>>>(psrc, pdst, plan->ld, plan->d, d_erow, d_col, e_lo, e_hi, d_w);
+        }
+        CLANE_LAUNCH_CHECK();
+    }
+    return clane_plan_softmax(plan, d_w, nullptr, d_rowptr, d_w, s);
+}
+
 int clane_cosine_finalize(const float* d_dots, const float* d_norms2, int64_t e, float* d_out, clane_stream_t s) {
     if (!d_dots || !d_norms2 || !d_out || e < 0) return CLANE_EINVAL;
     if (e == 0) return CLANE_OK;

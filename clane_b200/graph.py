@@ -27,6 +27,7 @@ import torch
 from torch.utils.data import Dataset
 
 from . import _lib
+from .similarity import AsymmertricSimilarity
 
 HUB_THRESHOLD = 0      # 0 = library default: rows longer than (edges of the plan / 4096), clamped to [256, 16384]
 
@@ -318,17 +319,33 @@ class Graph(Dataset):
             _lib.check(L.clane_build_p_cosine(S.plan.handle, Zc.data_ptr(), S.rowptr.data_ptr(), S.erow.data_ptr(),
                                               S.col.data_ptr(), S.w.data_ptr(), S.norms2.data_ptr(), stream),
                        "clane_build_p_cosine")
-        elif getattr(similarity, "_clane_kernel", None) == "asym" and L.clane_asym_supported(S.d) and S.e > 0:
-            # trainable bilinear scorer: every node projected once on the tensor cores, then per-edge dots + row softmax
+        elif (getattr(similarity, "_clane_kernel", None) == "asym" and S.e > 0
+              and type(similarity).forward is AsymmertricSimilarity.forward):
+            # trainable bilinear scorer: every node projected once on the tensor cores, then per-edge dots + row softmax.
+            # A subclass that overrides forward is scored by its own forward (the generic path below).
             if getattr(S, "asym_work", None) is None:
-                S.asym_work = torch.empty(2 * S.n * S.ld, dtype=torch.float32, device=S.device)
+                # P_src | P_dst, then the split of the stacked weights (the fp32 kernel's scratch)
+                S.asym_work = torch.zeros(2 * S.n * S.ld + 4 * S.d * S.ld, dtype=torch.float32, device=S.device)
                 S.asym_error = torch.zeros(1, dtype=torch.int32, device=S.device)
-            W = similarity.stacked_weights(S.device)
-            _lib.check(L.clane_build_p_asym(S.plan.handle, Zc.data_ptr(), W.data_ptr(), S.rowptr.data_ptr(), S.erow.data_ptr(),
-                                            S.col.data_ptr(), S.w.data_ptr(), S.asym_work.data_ptr(), S.asym_error.data_ptr(),
-                                            stream), "clane_build_p_asym")
+            S.asym_error.zero_()
+            if L.clane_asym_supported(S.d):
+                # d in {32, 64, 96, 128}: the TF32 kernel
+                name = "clane_build_p_asym"
+                W = similarity.stacked_weights(S.device)
+                rc = L.clane_build_p_asym(S.plan.handle, Zc.data_ptr(), W.data_ptr(), S.rowptr.data_ptr(), S.erow.data_ptr(),
+                                          S.col.data_ptr(), S.w.data_ptr(), S.asym_work.data_ptr(), S.asym_error.data_ptr(),
+                                          stream)
+            else:
+                # every other width: the fp32-faithful 3xTF32 kernel, W padded to rows of ld floats
+                name = "clane_build_p_asym_fp32"
+                W = torch.zeros([2 * S.d, S.ld], dtype=torch.float32, device=S.device)
+                W[:, :S.d] = similarity.stacked_weights(S.device)
+                rc = L.clane_build_p_asym_fp32(S.plan.handle, Zc.data_ptr(), W.data_ptr(), S.ld, S.rowptr.data_ptr(),
+                                               S.erow.data_ptr(), S.col.data_ptr(), S.w.data_ptr(), S.asym_work.data_ptr(),
+                                               S.asym_error.data_ptr(), stream)
+            _lib.check(rc, name)
             if int(S.asym_error.item()):          # synchronises: W must outlive the launch anyway
-                raise _lib.ClaneError("clane_build_p_asym: the projection kernel timed out waiting for its TMA copies")
+                raise _lib.ClaneError(f"{name}: the projection kernel timed out waiting for its TMA copies")
         else:
             # user plugin: honour its scores, still on the device; the softmax stays fused
             Zv = Zc[:S.n, :S.d]

@@ -7,6 +7,9 @@ Plugins are called as ``sim(v1, v2)`` with two ``[E, d]`` (or 1-D) tensors and r
 Built-in plugins carry ``_clane_kernel``; ``Graph.build_P`` dispatches on it to the fused
 per-edge score + neighbour-softmax kernels.  A user plugin without the tag is still honoured
 (its scores are computed by the plugin on device tensors, the softmax stays in CUDA).
+Precision of the fused scorers on fp32 embeddings: ``CosineSimilarity`` is bit-exact with the
+reference at every width; ``AsymmertricSimilarity`` reads TF32 at d in {32, 64, 96, 128} and is
+fp32-accurate (3xTF32) at every other width.
 """
 from __future__ import annotations
 
@@ -86,11 +89,16 @@ class AsymmertricSimilarity(nn.Module, Similarity):
 
     ``Phi_src`` / ``Phi_dst`` are bias-free ``nn.Linear(n_dim, n_dim)`` layers with Xavier-normal weights, as upstream
     (checkpoints and optimisers address them by these names).  A direct call scores pairs with torch on whatever device
-    the inputs live on.  ``Graph.build_P`` does not gather ``[E, d]`` rows for it: it hands the two weight matrices to
-    ``clane_build_p_asym``, which projects every NODE once on the tensor cores (tcgen05 tf32 GEMM, TMA-staged), takes the
-    per-edge dots of the projected rows and applies the row softmax -- for ``n_dim`` in {32, 64, 96, 128}; other widths go
-    through the generic plugin path.  The tensor-core inputs are TF32: scores agree with the fp32 module to ~1e-3 relative
-    (stated in tests/test_gpu_parity.py::test_asymmetric_scorer_fused_build_p)."""
+    the inputs live on.  ``Graph.build_P`` on fp32 embeddings does not gather ``[E, d]`` rows for it: it projects every
+    NODE once on the tensor cores (tcgen05 GEMM, TMA-staged), takes the per-edge dots of the projected rows and applies
+    the row softmax.  The precision depends on the width:
+      * ``n_dim`` in {32, 64, 96, 128}: ``clane_build_p_asym``, tensor-core inputs read as TF32 -- scores agree with the
+        fp32 module to ~1e-3 relative (tests/test_gpu_parity.py::test_asymmetric_scorer_fused_build_p);
+      * every other ``n_dim``: ``clane_build_p_asym_fp32``, 3xTF32 (each operand split into a TF32 part and its fp32
+        remainder) -- every projected value within (4 + 3 n_dim) 2^-23 sum_k |z_k w_k| of the exact product, i.e. fp32
+        accuracy (tests/test_asym_fp32.py).
+    Only this class's own ``forward`` is fused: a subclass that overrides it is scored by its ``forward`` on gathered
+    rows (the generic plugin path), as are fp64 embeddings."""
 
     _clane_kernel = "asym"
 

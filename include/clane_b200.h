@@ -194,6 +194,21 @@ int clane_asym_project(const float* d_Z, int32_t n, int32_t d, int32_t ld, const
 int clane_build_p_asym(clane_plan* plan, const float* d_Z, const float* d_W, const int32_t* d_rowptr, const int32_t* d_erow,
                        const int32_t* d_col, float* d_w, float* d_work, int32_t* d_error, clane_stream_t s);
 
+/* The same scorer at fp32 accuracy for any d >= 1 (3xTF32: each operand split into a TF32 high part and an fp32
+ * remainder, three tcgen05 MMAs per K step into one fp32 accumulator; every projected value lies within
+ * (4 + 3d) 2^-23 sum_k |z_k w_k| of the exact product).  d_W: the stacked weights [2d, ldw] row-major, ldw >= d a
+ * multiple of 4 (clane_padded_ld(d)), pad columns zero.  ld, ldw multiples of 4; d_Z and d_work 16-byte aligned.
+ * clane_asym_project_fp32: d_Psrc / d_Pdst [n, ld], only columns < d written; d_work: 4 * d * ldw floats (the split of W).
+ * clane_build_p_asym_fp32: projection, per-edge dots (the reference bmm's order: mul + add below d = 400, fma from there
+ * on), row softmax without the norm divisor; d_work: 2 * n * ld + 4 * d * ldw floats.
+ * Both return CLANE_EINVAL for a null pointer, d < 1, ld < d or ldw < d; *d_error is set to 1 if the kernel gave up
+ * waiting for its copies (it then writes no projected value). */
+int clane_asym_project_fp32(const float* d_Z, int32_t n, int32_t d, int32_t ld, const float* d_W, int32_t ldw, float* d_Psrc,
+                            float* d_Pdst, float* d_work, int32_t* d_error, clane_stream_t s);
+int clane_build_p_asym_fp32(clane_plan* plan, const float* d_Z, const float* d_W, int32_t ldw, const int32_t* d_rowptr,
+                            const int32_t* d_erow, const int32_t* d_col, float* d_w, float* d_work, int32_t* d_error,
+                            clane_stream_t s);
+
 /* The final division of CosineSimilarity.__call__ (similarity.py:37) for standalone plugin
  * calls: d_out[i] = d_dots[i] / fl(fl(sqrt(norms2[0])) * fl(sqrt(norms2[1]))).  May alias. */
 int clane_cosine_finalize(const float* d_dots, const float* d_norms2, int64_t e, float* d_out, clane_stream_t s);
