@@ -354,6 +354,10 @@ int clane_plan_create(clane_plan** out, int32_t n, int64_t e, int32_t d, const i
     clane_plan* plan = new (std::nothrow) clane_plan();
     if (!plan) return (int)cudaErrorMemoryAllocation;
     plan->n = n; plan->e = e; plan->d = d; plan->ld = clane_padded_ld(d);
+    // The kernels address rows of [n, ld] matrices by 32-bit unsigned float4 indices (the sweep's gathers and row
+    // pieces, the per-edge dots): n * ld <= 2^34 floats, 64 GiB per matrix.  A sweep at that bound would need 256 GiB
+    // for X and its three Z buffers, so the bound refuses no graph whose sweep fits a 180 GB device.
+    if ((int64_t)n * plan->ld > CLANE_MAX_MATRIX_FLOATS) { delete plan; return CLANE_ERANGE; }
     // Hub rows bound the critical path of a sweep: a row of k neighbours is an in-order chain of k/8 batches on
     // one warp (~150 ns per neighbour), so rows longer than 1/4096 of the edges this plan sweeps (a few percent of
     // the row kernel's duration) go to the segment + chain path.
@@ -376,7 +380,6 @@ int clane_plan_create(clane_plan** out, int32_t n, int64_t e, int32_t d, const i
     PLAN_CUDA(cudaMemset(plan->d_p2, 0, plan->p2_floats * sizeof(float)));
     if (!h_rowptr) { *out = plan; return CLANE_OK; }
 
-    if ((int64_t)n * plan->ld > (int64_t)INT32_MAX) { clane_plan_destroy(plan); return CLANE_ERANGE; }   // int32 row offsets
     plan->has_schedule = true;
     PLAN_CUDA(cudaMalloc(&plan->d_coloff, std::max<size_t>((size_t)e, 1) * sizeof(int32_t)));
     plan->row_lo = row_lo; plan->row_hi = row_hi;

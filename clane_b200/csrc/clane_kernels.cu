@@ -60,8 +60,12 @@ k_dots(const float* __restrict__ Za, const float* __restrict__ Zb, int ld, int d
     for (int64_t tile = (int64_t)blockIdx.x * dot_warps<kFma>() + warp; tile < ntiles; tile += (int64_t)gridDim.x * dot_warps<kFma>()) {
         const int64_t e0 = e_lo + tile * 32;
         const int cnt = (int)min((int64_t)32, e_hi - e0);
-        int ra = 0, rb = 0;                              // lane i: the two rows of edge e0 + i (float4 units)
-        if (lane < cnt) { ra = __ldg(erow + e0 + lane) * (ld >> 2); rb = __ldg(col + e0 + lane) * (ld >> 2); }
+        // lane i: the two rows of edge e0 + i as float4 indices, 32 bits unsigned (rows * ld <= 2^34, clane_plan_create)
+        unsigned ra = 0, rb = 0;
+        if (lane < cnt) {
+            ra = (unsigned)__ldg(erow + e0 + lane) * (unsigned)(ld >> 2);
+            rb = (unsigned)__ldg(col + e0 + lane) * (unsigned)(ld >> 2);
+        }
         float acc = 0.0f;
         for (int c0 = 0; c0 < d; c0 += kDotCols) {
             const int c = c0 + 4 * lane;
@@ -70,15 +74,15 @@ k_dots(const float* __restrict__ Za, const float* __restrict__ Zb, int ld, int d
             const float4* zd = reinterpret_cast<const float4*>(Zb) + (in ? c >> 2 : 0);
             // ---- phase A: 8 edges per round, 16 independent 128-bit loads in flight ----
             // (consecutive edges mostly share their source row -- CSR order: its piece is loaded once per run)
-            int prev = -1;
+            unsigned prev = ~0u;                         // no row starts there: (rows - 1) * ld / 4 < 2^32 - 1
             float4 xprev = make_float4(0.f, 0.f, 0.f, 0.f);
             for (int i = 0; i < cnt; i += 8) {
                 float4 x[8], y[8];
-                int oa[8];
+                unsigned oa[8];
 #pragma unroll
                 for (int u = 0; u < 8; ++u) {
                     oa[u] = __shfl_sync(kFull, ra, (i + u) & 31);
-                    const int ob = __shfl_sync(kFull, rb, (i + u) & 31);
+                    const unsigned ob = __shfl_sync(kFull, rb, (i + u) & 31);
                     y[u] = __ldg(zd + ob);
                     if (oa[u] != (u == 0 ? prev : oa[u - 1])) x[u] = __ldg(zc + oa[u]);     // uniform branch
                 }
@@ -269,10 +273,11 @@ k_row_softmax_long(const float* scores, const float* __restrict__ norms2, const 
     for (int i = tid; i < k; i += kSoftmaxLongThreads) w[a + i] = fmul(w[a + i], inv);
 }
 
-// col[e] * ld / 4: the float4 index the sweep gathers from (one multiply per edge, once per graph)
+// col[e] * ld / 4: the float4 index the sweep gathers from (one multiply per edge, once per graph), as uint32 bits:
+// n * ld <= 2^34 (clane_plan_create)
 __global__ void k_col_offsets(const int32_t* __restrict__ col, int64_t e, int ld, int32_t* __restrict__ off) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < e) off[i] = col[i] * (ld >> 2);
+    if (i < e) off[i] = (int32_t)((unsigned)col[i] * (unsigned)(ld >> 2));
 }
 
 __global__ void k_cosine_finalize(const float* __restrict__ dots, const float* __restrict__ norms2, int64_t e,

@@ -40,7 +40,7 @@ struct clane_plan {
     int32_t n_peers = 0, self_rank = 0;
     float* peers[3][16] = {};            // per Z buffer (two, or three when the caller rotates three): every rank's address
     float* mc[3] = {nullptr, nullptr, nullptr};   // multicast (NVLS) addresses of the two buffers, or null
-    int32_t* d_coloff = nullptr;       // col[e] * ld, rebuilt when the caller's column array changes
+    int32_t* d_coloff = nullptr;       // col[e] * ld / 4 as uint32 bits, rebuilt when the caller's column array changes
     const int32_t* coloff_src = nullptr;
     // CUDA-graph cache of enqueued sweep batches (all streams, all kernels): a propagate() call cycles through a few
     // argument sets (Z buffer rotation), so a handful of entries suffice; anything else evicts the oldest.

@@ -41,7 +41,7 @@ struct SweepParams {
     float* Zn;
     int ld, d, n;
     const int32_t* rowptr;
-    const int32_t* coloff;      // col[e] * ld / 4: float4 index of the neighbour's row
+    const int32_t* coloff;      // col[e] * ld / 4: float4 index of the neighbour's row, read as uint32 (n * ld <= 2^34)
     const float* w;
     float gamma;
     const SweepTask* tasks;     // sorted by work, descending (segments first)
@@ -381,9 +381,11 @@ __device__ __forceinline__ void run_span(const SweepParams& p, const int4 t0, in
             if (kBulk && run0 >= 0) { flush_rows(p, stage, r0, run0, r, lane); run0 = -1; }
             continue;
         }
-        const int row_off = (r0 + r) * p.ld + cc;          // n * ld < 2^31 (clane_plan_create)
-        cp_async16_sa(rowbuf_sa, p.X + row_off);
-        if (direct) cp_async16_sa(rowbuf_sa + 512, p.Zc + row_off);
+        // float4 index of the lane's piece of the row: 32 bits unsigned (n * ld <= 2^34, clane_plan_create), so the
+        // addresses below are IMAD.WIDE.U32 of one 32-bit register, as the gathers'
+        const unsigned row4 = (unsigned)(r0 + r) * (unsigned)(p.ld >> 2) + (unsigned)(cc >> 2);
+        cp_async16_sa(rowbuf_sa, reinterpret_cast<const float4*>(p.X) + row4);
+        if (direct) cp_async16_sa(rowbuf_sa + 512, reinterpret_cast<const float4*>(p.Zc) + row4);
         cp_async_commit();
         float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
         for (; k >= 8; k -= 8) {
@@ -411,9 +413,9 @@ __device__ __forceinline__ void run_span(const SweepParams& p, const int4 t0, in
             if (active) *reinterpret_cast<float4*>(stage + r * p.ld + cc) = out;
             if (run0 < 0) run0 = r;
         } else if (active) {
-            st_stream4(p.Zn + row_off, out);
-            if (p.mc != nullptr) multimem_st4(p.mc + row_off, out);
-            for (int j = 0; j < p.n_remote; ++j) *reinterpret_cast<float4*>(p.peer[j] + row_off) = out;
+            st_stream4(reinterpret_cast<float*>(reinterpret_cast<float4*>(p.Zn) + row4), out);
+            if (p.mc != nullptr) multimem_st4(reinterpret_cast<float*>(reinterpret_cast<float4*>(p.mc) + row4), out);
+            for (int j = 0; j < p.n_remote; ++j) reinterpret_cast<float4*>(p.peer[j])[row4] = out;
         }
         if (direct) {
             // the row is d / 32 consecutive cascade rows: transpose the float4-per-lane |delta| through 512 bytes of
@@ -638,7 +640,7 @@ __global__ void __launch_bounds__(kChainThreads, kLight ? 16 : 1) k_hub_chain(Sw
         lz[o] = 0.0f; lw[o] = 0.0f;
         if (o < nleft) {
             lw[o] = __ldg(p.w + a + nnb + o);
-            lz[o] = __ldg(p.Zc + (size_t)__ldg(p.coloff + a + nnb + o) * 4 + ccol);
+            lz[o] = __ldg(p.Zc + (size_t)(unsigned)__ldg(p.coloff + a + nnb + o) * 4 + ccol);
         }
     }
     if (blocked) {

@@ -120,6 +120,11 @@ class ShardedSweeper:
         if graph.X.dtype != torch.float32:
             raise NotImplementedError(f"sharded sweeps run in fp32 only; content embeddings are {graph.X.dtype} "
                                       "(use Embedder on one GPU for fp64)")
+        n_ld = graph._n * int(_lib.lib().clane_padded_ld(int(graph.X.shape[1])))
+        if n_ld >= 2 ** 31:
+            # the sharded exchange and its kernels are verified only below 2^31 elements per [N, ld] matrix
+            raise NotImplementedError(f"sharded sweeps need N*ld < 2^31; this graph has N*ld = {n_ld} "
+                                      "(use Embedder on one GPU for wider graphs)")
         self.g, self.sim, self.gamma = graph, similarity, float(np.float32(gamma))
         self.world, self.rank = dist.get_world_size(), dist.get_rank()
         self.dev = _lib.require_cuda()

@@ -37,7 +37,7 @@ extern "C" {
 
 #define CLANE_OK 0
 #define CLANE_EINVAL (-1)      /* bad argument (null pointer, negative size, d < 1 ...) */
-#define CLANE_ERANGE (-2)      /* edge endpoint outside [0, n) / size exceeds int32 indexing */
+#define CLANE_ERANGE (-2)      /* edge endpoint outside [0, n) / n or e >= 2^31 / n * ld > CLANE_MAX_MATRIX_FLOATS */
 #define CLANE_EWORKSPACE (-3)  /* caller-provided buffer too small */
 #define CLANE_ENODEVICE (-4)   /* no CUDA device / not an sm_100 class device */
 #define CLANE_ENOENT (-5)      /* file cannot be opened */
@@ -109,8 +109,12 @@ int clane_edges_close(clane_edge_file* f);
  * hub_threshold <= 0 selects the default: (edges of rows [row_lo, row_hi)) / 4096 rounded up to a
  * multiple of 8, clamped to [256, 16384] (a row is an in-order chain on one warp; this bounds it
  * to a few percent of a sweep).
- * h_rowptr may be NULL for a scores-only plan (clane_scores_cosine / clane_l1_*). */
+ * h_rowptr may be NULL for a scores-only plan (clane_scores_cosine / clane_l1_*).
+ * Every plan, scores-only included, needs n * clane_padded_ld(d) <= CLANE_MAX_MATRIX_FLOATS
+ * (CLANE_ERANGE otherwise): the fp32 kernels address the rows of an [n, ld] matrix by 32-bit
+ * unsigned float4 indices. */
 typedef struct clane_plan clane_plan;
+#define CLANE_MAX_MATRIX_FLOATS (1LL << 34)   /* 64 GiB of fp32 per [n, ld] matrix */
 /* The schedule alone, on the host (what clane_plan_create uploads); every output has capacity
  * row_hi - row_lo + 1.
  *   spans       : runs of consecutive ordinary rows inside one group holding at most
