@@ -596,72 +596,6 @@ def test_asymmetric_scorer_fused_build_p(n, d):
     assert L.clane_asym_supported(100) == 0 and L.clane_asym_supported(128) == 1
 
 
-def test_peer_stores_and_value_finish_single_gpu():
-    """The fused exchange on one GPU: a plan over half of the rows, with a second local buffer registered as the
-    'peer' -- after the sweep the peer holds exactly the swept rows (ordinary, paired, hub), nothing else; and the
-    finish from all-reduced values (clane_l1_tail_values + clane_l1_finish_values) equals clane_l1_diff."""
-    L = _lib.lib()
-    rng = np.random.default_rng(21)
-    for n, d in [(6000, 128), (3000, 100)]:
-        src, dst = synth.make_edges(n, n * 6, "powerlaw", rng)
-        src = np.concatenate([src, np.full(700, 17)])            # one row long enough for the segment + chain path
-        dst = np.concatenate([dst, rng.permutation(n)[:700]])
-        X = rng.standard_normal((n, d), dtype=np.float32)
-        g = Graph.from_arrays(n, src, dst, X)
-        S = g._device_state()
-        g._build_P_device(similarity.CosineSimilarity())
-        lo, hi = 0, (n // 2) // 8 * 8
-        plan = _lib.Plan(n, g._nnz, d, g._rowptr, lo, hi, 0)
-        assert plan.n_hub_rows >= 1
-        zn = S.Z[1].clone()
-        peer = torch.full_like(zn, -7.0)
-        own = (ctypes.c_uint64 * 2)(zn.data_ptr(), peer.data_ptr())
-        other = (ctypes.c_uint64 * 2)(peer.data_ptr(), zn.data_ptr())       # the second ping-pong buffer: unused here
-        _lib.check(L.clane_plan_set_peers(plan.handle, 2, 0, own, other))
-        s = _lib.stream_handle()
-        _lib.check(L.clane_sweep(plan.handle, S.X.data_ptr(), S.Z[0].data_ptr(), zn.data_ptr(), S.rowptr.data_ptr(),
-                                 S.col.data_ptr(), S.w.data_ptr(), ctypes.c_float(0.76), 0, 0, 0, 0, s))
-        torch.cuda.synchronize()
-        deg = np.diff(g._rowptr)
-        swept = np.zeros(n, bool)
-        swept[lo:hi] = deg[lo:hi] > 0
-        zn_h, peer_h = zn.cpu().numpy(), peer.cpu().numpy()
-        assert np.array_equal(peer_h[swept], zn_h[swept])
-        assert np.all(peer_h[~swept] == -7.0)
-        # reference values of the swept rows: the full single-GPU sweep
-        full = S.Z[1].clone()
-        _lib.check(L.clane_sweep(S.plan.handle, S.X.data_ptr(), S.Z[0].data_ptr(), full.data_ptr(), S.rowptr.data_ptr(),
-                                 S.col.data_ptr(), S.w.data_ptr(), ctypes.c_float(0.76), 0, 0, 0, 0, s))
-        torch.cuda.synchronize()
-        assert np.array_equal(full.cpu().numpy()[swept], zn_h[swept])
-        # a third rotating buffer (clane_plan_set_peers_third): a sweep into it reaches its own peer copy, not the others'
-        z3, peer3 = S.Z[1].clone(), torch.full_like(zn, -9.0)
-        third = (ctypes.c_uint64 * 2)(z3.data_ptr(), peer3.data_ptr())
-        _lib.check(L.clane_plan_set_peers_third(plan.handle, third))
-        peer.fill_(-7.0)
-        _lib.check(L.clane_sweep(plan.handle, S.X.data_ptr(), S.Z[0].data_ptr(), z3.data_ptr(), S.rowptr.data_ptr(),
-                                 S.col.data_ptr(), S.w.data_ptr(), ctypes.c_float(0.76), 0, 0, 0, 0, s))
-        torch.cuda.synchronize()
-        assert np.array_equal(peer3.cpu().numpy()[swept], zn_h[swept]) and np.all(peer3.cpu().numpy()[~swept] == -9.0)
-        assert np.all(peer.cpu().numpy() == -7.0)
-        # value-based finish == clane_l1_diff
-        nodes = ctypes.c_int64()
-        _lib.check(L.clane_cascade_shape(n * d, ctypes.byref(nodes), None))
-        k = nodes.value
-        p1 = torch.zeros((k + 3) * 32, device="cuda")
-        vals = p1[(k + 2) * 32:]
-        _lib.check(L.clane_l1_partial(S.plan.handle, full.data_ptr(), S.Z[0].data_ptr(), 0, k, p1.data_ptr(), s))
-        _lib.check(L.clane_l1_tail_values(S.plan.handle, full.data_ptr(), S.Z[0].data_ptr(), vals.data_ptr(), s))
-        out = torch.zeros(2, device="cuda")
-        _lib.check(L.clane_l1_finish_values(S.plan.handle, p1.data_ptr(), vals.data_ptr(), out.data_ptr(), 0, 0, 0, s))
-        _lib.check(L.clane_l1_diff(S.plan.handle, full.data_ptr(), S.Z[0].data_ptr(), out[1:].data_ptr(), s))
-        o = out.cpu().numpy()
-        assert o[0] == o[1] and o[0] > 0
-    assert L.clane_plan_set_peers(plan.handle, 17, 0, own, other) == -1
-    assert L.clane_plan_set_peers(plan.handle, 2, 2, own, other) == -1
-    _lib.check(L.clane_plan_set_peers(plan.handle, 0, 0, None, None))
-
-
 @pytest.mark.parametrize("n,d", [(7, 1), (5, 3), (33, 5), (1000, 7)])
 def test_value_finish_small_and_ragged(n, d):
     """n*d < 8 (ATen's scalar path), and ragged tails: the values the finish needs come from the 32-float buffer."""
